@@ -1,13 +1,15 @@
 #!/usr/bin/env python
 """bench.py — decoded coded Gb/s of the LDPC decode hot path on B200 (contract: see DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, NCCL)
 
 Headline workload (BASELINE.json configs[1]): codes/ref_h_n1152_m1024.txt (n=1024, k=128 transmitted), AWGN,
 BP_MS, -i 50, every frame running the full 50 iterations (the "@50 iters" of the metric, i.e. --no-early-term).  One
 step = one pass of channel -> decode -> accounting over FRAMES_PER_STEP frames per GPU (weak scaling: frames shard
-over GPUs, counters are all-reduced once per step).
+over GPUs, counters are all-reduced once per step).  --dump-outputs DIR writes what the last timed step returned to its
+caller, the counters {frame errors, bit errors, frames, sum of reference iteration counts, sum of executed iterations}
+over all GPUs, as DIR/counters.npy (float64); the frames of every step are fixed by the seed and the step index.
 
 Besides the headline the line carries (N=1): `configs` — all five BASELINE.json configurations, each device-timed with
 its own roofline (shared memory / HBM / FP64 pipe); `e2e` — the batch decode call with HOST buffers; `cpu_baseline` — the
@@ -19,6 +21,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -189,7 +192,8 @@ def boxplus_per_iteration(nnz, mc):
 def run_configs(api, smem_peak, fp64_peak, hbm_peak, traffic):
     sys.path.insert(0, os.path.join(ROOT, "codes"))
     import gen_codes
-    big = gen_codes.ensure()
+    codes_dir = tempfile.TemporaryDirectory()      # generated outside the tree, which may be read-only
+    big = gen_codes.ensure(directory=codes_dir.name)
     out = {}
 
     def measure(ctx, channel, xs, decoding, et, frames, reps=2):
@@ -275,6 +279,7 @@ def run_configs(api, smem_peak, fp64_peak, hbm_peak, traffic):
     entry("C4_dvbs2_bp_noet", ctx, ms, fr, ed, st, "hbm", "configs[3] DVB-S2-shaped IRA code n=64800 r=1/2 (nnz 226799), AWGN +1 dB, BP fp64, --no-early-term",
           fp64_block(ctx, ed, ms, "C4_dvbs2_bp_noet"))
     ctx.close()
+    codes_dir.cleanup()
     return out, launches
 
 
@@ -348,13 +353,15 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     step_cnt = torch.zeros(8, dtype=torch.int64, device="cuda")
+    last_cnt = torch.zeros(8, dtype=torch.int64, device="cuda")   # the last timed step's counters (--dump-outputs)
 
-    def step(i, early_term=False):
-        """one pass of channel -> decode -> accounting over this rank's n_step frames (+ the counter all-reduce when sharded)"""
+    def step(i, early_term=False, last=False):
+        """one pass of channel -> decode -> accounting over this rank's n_step frames (+ the counter all-reduce when sharded);
+        last: the step's counters go to last_cnt as well (world > 1) or instead of counters (world == 1)"""
         frame0 = (i * world + rank) * n_step
         if world == 1:
-            ctx.sim_point_async(counters.data_ptr(), stream.cuda_stream, "AWGN", SNR_DB, seed=0, point=0, frame0=frame0, nframes=n_step,
-                                decoding=DECODING, iterations=ITERS, early_term=early_term)
+            ctx.sim_point_async((last_cnt if last else counters).data_ptr(), stream.cuda_stream, "AWGN", SNR_DB, seed=0, point=0,
+                                frame0=frame0, nframes=n_step, decoding=DECODING, iterations=ITERS, early_term=early_term)
             return
         with torch.cuda.stream(stream):
             step_cnt.zero_()
@@ -362,13 +369,15 @@ def run_ours(args):
                                 decoding=DECODING, iterations=ITERS, early_term=early_term)
             dist.all_reduce(step_cnt)        # 64 B over NVLink: the only collective of the path
             counters.add_(step_cnt)
+            if last:
+                last_cnt.copy_(step_cnt)
 
-    def timed(nsteps, first, early_term=False):
+    def timed(nsteps, first, early_term=False, keep_last=False):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record(stream)
         for i in range(nsteps):
-            step(first + i, early_term)
+            step(first + i, early_term, last=keep_last and i == nsteps - 1)
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
@@ -386,13 +395,20 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(args.steps, 0)
+    ms = timed(args.steps, 0, keep_last=True)
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.stats()["launches"]
     total_frames = n_step * world * args.steps
     value = total_frames * NCT / (ms * 1e-3) / 1e9
+    if world == 1:
+        counters.add_(last_cnt)
     cnt = counters.cpu().tolist()
     assert cnt[2] == total_frames, (cnt, total_frames)   # every frame of every rank was decoded and counted
+    last = last_cnt.cpu().numpy()[:5]
+    assert last[2] == n_step * world, last
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "counters.npy"), last.astype(np.float64))
 
     # per-launch duration of the dominant kernel (single launch per step) with events on the launch stream
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -598,8 +614,11 @@ def main():
     ap.add_argument("--steps", type=int, default=6)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -152,12 +152,13 @@ def dvbs2_like_r12(path=DVBS2_FILE, seed=302307):
     return _write(path, m, n, rows, cols)
 
 
-def ensure(which=("bg1", "dvbs2")):
+def ensure(which=("bg1", "dvbs2"), directory=HERE):
+    """Paths of the code files in `directory`; the missing ones are generated there."""
     out = {}
-    if "bg1" in which:
-        out["bg1"] = BG1_FILE if os.path.exists(BG1_FILE) else nr_bg1_like()
-    if "dvbs2" in which:
-        out["dvbs2"] = DVBS2_FILE if os.path.exists(DVBS2_FILE) else dvbs2_like_r12()
+    for name, default, make in (("bg1", BG1_FILE, nr_bg1_like), ("dvbs2", DVBS2_FILE, dvbs2_like_r12)):
+        if name in which:
+            path = os.path.join(directory, os.path.basename(default))
+            out[name] = path if os.path.exists(path) else make(path)
     return out
 
 

@@ -1,3 +1,4 @@
+import functools
 import os
 import sys
 
@@ -18,6 +19,43 @@ def large_code_files():
     sys.path.insert(0, os.path.join(ROOT, "codes"))
     import gen_codes
     return gen_codes.ensure()
+
+
+LARGE_REF = os.path.join(GOLDEN, "large_codes_ref.npz")   # written by tests/golden/make_large_golden.py
+
+
+def large_case_key(name, llr, decoding, iters, et):
+    """Names one decode of the large codes by its inputs: code, decoder settings and a digest of the LLRs."""
+    import hashlib
+    import numpy as np
+    digest = hashlib.sha256(np.ascontiguousarray(llr, dtype=np.float64).tobytes()).hexdigest()[:16]
+    return "%s:%s:%d:%d:%s" % (name, decoding, iters, int(et), digest)
+
+
+@functools.lru_cache(maxsize=None)
+def _large_ref_cases():
+    return _load_cases(LARGE_REF)
+
+
+def reference_outputs(name, path, oc, llr, decoding, iters, et):
+    """The reference decoder's outputs on the large codes: the oracle's full outputs, checked against what the unmodified
+    reference decoder (its ldpc_decoder::decode through oracle/dump_ref.cpp) returned for the same inputs.  Stored per
+    case: iteration counts, hard decisions, a SHA-256 of the posterior LLRs' bytes and a fixed sample of them."""
+    import hashlib
+    import numpy as np
+    cases = _large_ref_cases()
+    with open(path, "rb") as f:
+        assert hashlib.sha256(f.read()).hexdigest() == str(cases["code_" + name]["sha256"]), \
+            "%s differs from the code file the reference outputs were recorded on (codes/gen_codes.py)" % path
+    key = large_case_key(name, llr, decoding, iters, et)
+    assert key in cases, "no stored reference outputs for %s: regenerate with tests/golden/make_large_golden.py" % key
+    ref = cases[key]
+    out, co, its = oc.decode(llr, iters, et, decoding == "BP_MS")
+    assert np.array_equal(its, ref["iters"]), key
+    assert np.array_equal(np.packbits(co, axis=1), ref["co_bits"]), key
+    assert np.array_equal(out[:, ref["sample_idx"]].view(np.uint64), ref["llr_out_sample"].view(np.uint64)), key
+    assert hashlib.sha256(out.tobytes()).hexdigest() == str(ref["llr_out_sha256"]), key
+    return out, co, its
 
 
 def pytest_configure(config):
