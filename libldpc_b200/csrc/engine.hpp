@@ -3,8 +3,10 @@
 // touched lazily so that loader / GF(2) helpers work on machines without a GPU.
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <map>
 #include <memory>
+#include <set>
 #include <string>
 #include <tuple>
 #include <vector>
@@ -12,8 +14,28 @@
 #include "../../include/ldpc_b200.h"
 #include "code.hpp"
 
+struct CUevent_st;  // cudaEvent_t = CUevent_st *
+struct CUstream_st; // cudaStream_t = CUstream_st *
+
 namespace b200
 {
+    // Owners of CUDA resources; the deleters are defined in engine.cu, and ignore errors as teardown has nobody to report to.
+    struct DeviceFree { void operator()(void *p) const; };
+    struct PinnedFree { void operator()(void *p) const; };
+    struct EventDestroy { void operator()(CUevent_st *e) const; };
+    struct StreamDestroy { void operator()(CUstream_st *s) const; };
+    template <typename T>
+    using DevPtr = std::unique_ptr<T, DeviceFree>;    // device memory (cudaMalloc)
+    template <typename T>
+    using PinnedPtr = std::unique_ptr<T, PinnedFree>; // pinned host memory (cudaHostAlloc)
+    using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+    using Stream = std::unique_ptr<CUstream_st, StreamDestroy>;
+    struct DevBuf // device buffer that is grown on demand
+    {
+        DevPtr<unsigned char> p;
+        size_t cap = 0; // bytes
+    };
+
     struct DeviceLayered;    // device-resident LayeredLayout (engine.cu; layered schedule)
     struct DeviceLayout;     // device-resident TileLayout (engine.cu; erasure decoder)
     struct DeviceSegLayout;  // device-resident SegLayout (engine.cu; tile4 kernel)
@@ -104,7 +126,7 @@ namespace b200
         double fp64_probe();
 
         void ensure_cuda();
-        void *engine_stream() const { return stream_; }
+        void *engine_stream() const { return stream_.get(); }
 
     private:
         struct Config
@@ -120,9 +142,14 @@ namespace b200
         const SegLayout &get_seg_layout(int lanes, int threads, int isz = 4);
         DeviceSegLayout &device_seg_layout(int lanes, int threads, int isz = 4);
         const TileLayout &get_layout(int fpc, int threads);
-        void autotune_global(int alg, const decoder_param &dp, void *stream);
-        void autotune_pair(int alg, const decoder_param &dp, void *stream);
-        void maybe_autotune(int alg, const decoder_param &dp, uint64_t n_frames, void *stream);
+        struct TrialGuard; // puts back what a shape trial changes (engine.cu)
+        void autotune_global(int alg, const decoder_param &dp, CUstream_st *s);
+        void autotune_pair(int alg, const decoder_param &dp, CUstream_st *s);
+        // one shape trial: frames per ms of the current shape on synthetic AWGN frames; 0 when it is not a candidate
+        double trial_rate(const decoder_param &dp, double snr, unsigned long long *d_cnt, uint64_t frames, CUstream_st *s,
+                          const std::function<bool()> &eligible = nullptr);
+        float time_ms(CUstream_st *s, const std::function<void()> &work); // device time of `work` on s (ev0_ .. ev1_; blocking)
+        void maybe_autotune(int alg, const decoder_param &dp, uint64_t n_frames, CUstream_st *s);
         // outcomes of the shape trials are remembered across processes: $LDPC_B200_TUNE_CACHE (a directory; "off" disables) or
         // ~/.cache/libldpc_b200, one small text file per (code, device)
         std::string tune_cache_file();
@@ -130,55 +157,62 @@ namespace b200
         void tune_cache_store();
         bool tune_cache_loaded_ = false;
         std::string device_name_;
-        void launch_layered(const decoder_param &dp, const FrameSource &src, const FrameSink &sink, uint64_t n_frames, void *stream);
+        void launch_layered(const decoder_param &dp, const FrameSource &src, const FrameSink &sink, uint64_t n_frames, CUstream_st *s);
         std::vector<std::vector<int>> layers_;
         std::map<std::pair<int, int>, std::unique_ptr<LayeredLayout>> lay_layouts_;
-        std::map<std::pair<int, int>, std::unique_ptr<DeviceLayered>> dev_lay_;
-        void launch_bec(const decoder_param &dp, const FrameSource &src, const FrameSink &sink, uint64_t n_frames, void *stream);
+        void launch_bec(const decoder_param &dp, const FrameSource &src, const FrameSink &sink, uint64_t n_frames, CUstream_st *s);
         DeviceLayout &device_layout(int fpc, int threads, bool idx16);
-        void ensure_state(size_t bytes, void *stream);
-        void release_state(void *stream);
+        void ensure_state(size_t bytes, CUstream_st *s);
+        void release_state(CUstream_st *s);
         bool try_seg_layout(int lanes, int threads, int isz);
         static int channel_kind(const std::string &name);
+        const void *tile_fn(const Config &c, bool et); // the tile kernel of c (early termination: et), its attributes set
+        // dynamic shared-memory opt-in (max_shared: and the all-shared carveout) of a kernel, set on this engine's first use of it
+        void set_smem_attributes(const void *fn, int smem_optin, bool max_shared);
+        std::set<const void *> attrs_set_; // kernels whose attributes this engine has set (it is bound to one device)
+        // stats of the last launch, and of a finished job (from its counters)
+        void note_launch(int fpc, int threads, int ctas, int residency, int precision, size_t smem_bytes);
+        void account(double ms, uint64_t frames, uint64_t executed_iterations);
 
         bool cuda_ready_ = false;
         int sm_count_ = 148;
         size_t smem_optin_ = 227 * 1024, smem_per_sm_ = 228 * 1024;
         std::map<std::pair<int, int>, int> pair_tuned_; // (precision, alg) -> 1 when the two-CTAs-per-SM shape won its trial (shared-memory residency)
         int force_pair_ = -1;                           // trial: -1 = use pair_tuned_, 0/1 = force
-        void *stream_ = nullptr;
-        void *ev0_ = nullptr, *ev1_ = nullptr;
         std::map<std::pair<int, int>, std::unique_ptr<TileLayout>> layouts_;
-        std::map<std::tuple<int, int, bool>, std::unique_ptr<DeviceLayout>> dev_layouts_;
         std::map<std::tuple<int, int, int>, std::unique_ptr<SegLayout>> seg_layouts_;
-        std::map<std::tuple<int, int, int>, std::unique_ptr<DeviceSegLayout>> dev_seg_layouts_;
         std::map<std::tuple<int, int, int, int, int, size_t>, int> occupancy_;
         std::map<std::pair<int, int>, std::tuple<int, int, int>> tuned_; // (precision, alg) -> autotuned (lanes, threads, wide), global residency
         bool in_autotune_ = false;
         int force_wide_ = -1; // autotune trials: -1 = use tuned_/default, 0/1 = force
-        int32_t *d_bit_pos_ = nullptr, *d_punct_ = nullptr, *d_short_ = nullptr;
-        int32_t *d_g_col_ptr_ = nullptr, *d_g_row_ = nullptr; // generator matrix by column (device)
-        int32_t *d_bs_row_ptr_ = nullptr, *d_bs_col_ptr_ = nullptr; // bit-sliced BEC kernel
-        uint16_t *d_bs_row_slot_ = nullptr, *d_bs_col_slot_ = nullptr;
         std::unique_ptr<BecSliceLayout> bs_layout_;
-        uint8_t *d_bs_tx_flag_ = nullptr;
-        unsigned long long *d_counters_ = nullptr;
-        double *d_ask_X_ = nullptr;
-        int32_t *d_ask_label_ = nullptr, *d_ask_rev_ = nullptr, *d_ask_bm_ = nullptr;
-        bool ask_uploaded_ = false;
         void ask_fill(void *ask_params); // uploads the tables on first use and fills an AskParams
-        unsigned long long *d_round_[2] = {nullptr, nullptr}, *h_round_[2] = {nullptr, nullptr}; // sweep rounds in flight
-        void *ev_round_[2] = {nullptr, nullptr}, *ev_round0_[2] = {nullptr, nullptr}, *ev_rdone_[2] = {nullptr, nullptr};
-        unsigned char *d_state_ = nullptr;
-        size_t state_bytes_ = 0;
-        void *ev_state_ = nullptr; // recorded after every launch that uses the state block
         bool state_used_ = false;
+
+        // CUDA resources.  Members are destroyed in reverse order: device layouts first, then buffers and events, then the
+        // copy streams, and the engine stream last.
+        Stream stream_;
+        Event ev0_, ev1_;
         // host-buffer batch decode pipeline (decode_batch_host): copy streams, per-buffer events, cached device buffers
-        void *copy_in_ = nullptr, *copy_out_ = nullptr;
-        void *ev_in_[2] = {nullptr, nullptr}, *ev_k_[2] = {nullptr, nullptr}, *ev_out_[2] = {nullptr, nullptr};
-        void *db_in_[2] = {nullptr, nullptr}, *db_out_[2] = {nullptr, nullptr}, *db_hard_[2] = {nullptr, nullptr}, *db_it_[2] = {nullptr, nullptr};
-        void *db_bits_[2] = {nullptr, nullptr};
-        size_t db_in_cap_[2] = {0, 0}, db_out_cap_[2] = {0, 0}, db_hard_cap_[2] = {0, 0}, db_it_cap_[2] = {0, 0}, db_bits_cap_[2] = {0, 0};
+        Stream copy_in_, copy_out_;
+        Event ev_in_[2], ev_k_[2], ev_out_[2];
+        DevBuf db_in_[2], db_out_[2], db_hard_[2], db_it_[2], db_bits_[2];
+        DevPtr<unsigned long long> d_round_[2]; // sweep rounds in flight
+        PinnedPtr<unsigned long long> h_round_[2];
+        Event ev_round_[2], ev_round0_[2], ev_rdone_[2];
+        DevBuf state_;  // per-CTA state block (ensure_state)
+        Event ev_state_; // recorded after every launch that uses the state block
+        DevPtr<int32_t> d_bit_pos_, d_punct_, d_short_;
+        DevPtr<int32_t> d_g_col_ptr_, d_g_row_; // generator matrix by column (device)
+        DevPtr<int32_t> d_bs_row_ptr_, d_bs_col_ptr_; // bit-sliced BEC kernel
+        DevPtr<uint16_t> d_bs_row_slot_, d_bs_col_slot_;
+        DevPtr<uint8_t> d_bs_tx_flag_;
+        DevPtr<unsigned long long> d_counters_;
+        DevPtr<double> d_ask_X_;
+        DevPtr<int32_t> d_ask_label_, d_ask_rev_, d_ask_bm_;
+        std::map<std::tuple<int, int, bool>, std::unique_ptr<DeviceLayout>> dev_layouts_;
+        std::map<std::tuple<int, int, int>, std::unique_ptr<DeviceSegLayout>> dev_seg_layouts_;
+        std::map<std::pair<int, int>, std::unique_ptr<DeviceLayered>> dev_lay_;
     };
 
     // reference-semantics sweep driver (sim_driver.cpp)

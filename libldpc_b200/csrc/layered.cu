@@ -1,40 +1,18 @@
 // layered-schedule kernel instantiations (layered.cuh)
 #include <stdexcept>
-#include <string>
 
 #include "layered.cuh"
 
 namespace b200
 {
-    template <typename T, int ALG, int LANES>
-    static void launch_one(const LayParams &p, int ctas, int threads, cudaStream_t s)
+    const void *layered_kernel(bool f32, int alg, int lanes)
     {
-        lay_kernel<T, ALG, LANES><<<ctas, threads, 0, s>>>(p);
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e) + " (layered kernel launch)");
+        static const void *const kernels[2][2][2] = {
+            {{(const void *)lay_kernel<double, ALG_MS, 2>, (const void *)lay_kernel<double, ALG_MS, 4>},
+             {(const void *)lay_kernel<double, ALG_BP, 2>, (const void *)lay_kernel<double, ALG_BP, 4>}},
+            {{(const void *)lay_kernel<float, ALG_MS, 2>, (const void *)lay_kernel<float, ALG_MS, 4>},
+             {(const void *)lay_kernel<float, ALG_BP, 2>, (const void *)lay_kernel<float, ALG_BP, 4>}}};
+        if (lanes != 2 && lanes != 4) throw std::runtime_error("layered schedule: lanes per node must be 2 or 4");
+        return kernels[f32][alg == ALG_BP][lanes == 4];
     }
-    template <typename T, int ALG>
-    void run_layered_kernel(const LayParams &p, int lanes, int ctas, int threads, cudaStream_t s)
-    {
-        if (lanes == 2) launch_one<T, ALG, 2>(p, ctas, threads, s);
-        else if (lanes == 4) launch_one<T, ALG, 4>(p, ctas, threads, s);
-        else throw std::runtime_error("layered schedule: lanes per node must be 2 or 4");
-    }
-    template <typename T, int ALG>
-    int layered_occupancy(int lanes, int threads)
-    {
-        int n = 0;
-        cudaError_t e = lanes == 2 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, lay_kernel<T, ALG, 2>, threads, 0)
-                                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, lay_kernel<T, ALG, 4>, threads, 0);
-        if (e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e));
-        return n;
-    }
-    template void run_layered_kernel<double, ALG_MS>(const LayParams &, int, int, int, cudaStream_t);
-    template void run_layered_kernel<double, ALG_BP>(const LayParams &, int, int, int, cudaStream_t);
-    template void run_layered_kernel<float, ALG_MS>(const LayParams &, int, int, int, cudaStream_t);
-    template void run_layered_kernel<float, ALG_BP>(const LayParams &, int, int, int, cudaStream_t);
-    template int layered_occupancy<double, ALG_MS>(int, int);
-    template int layered_occupancy<double, ALG_BP>(int, int);
-    template int layered_occupancy<float, ALG_MS>(int, int);
-    template int layered_occupancy<float, ALG_BP>(int, int);
 } // namespace b200

@@ -382,8 +382,6 @@ namespace b200
         if (tid < 5 && s_cnt[tid]) atomicAdd(&p.counters[tid], s_cnt[tid]);
     }
 
-    template <typename T, int ALG>
-    void run_layered_kernel(const LayParams &p, int lanes, int ctas, int threads, cudaStream_t s);
-    template <typename T, int ALG>
-    int layered_occupancy(int lanes, int threads);
+    // the layered kernel for (precision, algorithm, lanes per node: 2 or 4); layered.cu instantiates them
+    const void *layered_kernel(bool f32, int alg, int lanes);
 } // namespace b200

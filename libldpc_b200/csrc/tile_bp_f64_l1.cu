@@ -2,5 +2,5 @@
 #include "tile_launch.cuh"
 namespace b200
 {
-    B200_DEFINE_TILE_LANES(double, ALG_BP, 1)
+    template const void *tile_variant<double, ALG_BP, 1>(bool, bool, bool, bool, bool);
 }

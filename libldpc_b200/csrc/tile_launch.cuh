@@ -1,119 +1,58 @@
-// Launch front end of the tile kernel family.  Each (T, ALG) pair is instantiated in its own
-// translation unit (tile_*.cu) so that the build can compile them in parallel.
+// Variant choice of the tile kernel family.  Each (T, ALG, lanes) is instantiated in its own translation unit
+// (tile_<alg>_<prec>_l<lanes>.cu) so that the build can compile them in parallel.
 #pragma once
-#include <atomic>
-#include <cuda_runtime.h>
 #include <stdexcept>
-#include <string>
 
 #include "tile4.cuh"
 
 namespace b200
 {
+    constexpr int TILE_SMEM_OPTIN = 232448 - 2048; // 227 KB minus the kernel's static shared memory (scheduling state, a copy of the arguments)
+
     // Variants per (T, ALG, lanes): shared-memory residency with the TMEM mirror (with / without the
     // early-termination syndrome: --no-early-term min-sum runs skip it), shared-memory residency without the mirror,
     // global residency (min-sum: a narrow 2-CTA/64-register and a wide 1-CTA/128-register build).  Index entries are
-    // 32-bit byte offsets.
+    // 32-bit byte offsets, or 16-bit with the TMEM mirror (idx16).
     // lanes = warp lanes per node (frames per CTA = lanes * 16/sizeof(T)).
-
-    constexpr int TILE_SMEM_OPTIN = 232448 - 2048; // 227 KB minus the kernel's static shared memory (scheduling state, a copy of the arguments)
-
-    template <typename T, typename IdxT, int ALG, bool SMEM, int LANES, bool TM, bool ET, int MINB>
-    void prepare_tile_one()
-    {
-        // the opt-in is a per-device attribute of the function: remember it per device (several GPUs in one process)
-        static std::atomic<bool> attr_set[64];
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (dev < 0 || dev >= 64 || !attr_set[dev].load(std::memory_order_acquire))
-        {
-            cudaError_t e = cudaFuncSetAttribute(tile4_kernel<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN);
-            if (e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e));
-            // all of the L1/shared array as shared memory: the shared-memory kernels keep their working set there (two CTAs per
-            // SM need it); the global-residency kernels keep the default split, they live off the L1 cache
-            if constexpr (SMEM) cudaFuncSetAttribute(tile4_kernel<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            if (dev >= 0 && dev < 64) attr_set[dev].store(true, std::memory_order_release);
-        }
-    }
-
-    template <typename T, typename IdxT, int ALG, bool SMEM, int LANES, bool TM, bool ET, int MINB>
-    void launch_tile_one(const K4Params &kp, int ctas, int threads, size_t smem_bytes, cudaStream_t s)
-    {
-        prepare_tile_one<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB>();
-        tile4_kernel<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB><<<ctas, threads, smem_bytes, s>>>(kp);
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e) + " (tile kernel launch)");
-    }
-
-    template <typename T, typename IdxT, int ALG, bool SMEM, int LANES, bool TM, bool ET, int MINB>
-    int occupancy_tile_one(int threads, size_t smem_bytes)
-    {
-        prepare_tile_one<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB>();
-        int n = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, tile4_kernel<T, IdxT, ALG, SMEM, LANES, TM, ET, MINB>, threads, smem_bytes);
-        if (e != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e));
-        return n;
-    }
-
-    // One translation unit per (T, ALG, lanes) — tile_<alg>_<prec>_l<lanes>.cu — so that the build compiles the kernel
-    // variants in parallel; engine.cu holds the dispatch over `lanes`.
     // wide (global residency, min-sum): the 1-CTA-per-SM / 128-register build instead of the 2-CTA / 64-register one
     template <typename T, int ALG, int L>
-    void launch_tile_lanes(const K4Params &kp, bool smem, bool tm, bool et, bool wide, bool idx16, int ctas, int threads, size_t smem_bytes, cudaStream_t s);
-    template <typename T, int ALG, int L>
-    int occupancy_tile_lanes(bool smem, bool tm, bool et, bool wide, bool idx16, int threads, size_t smem_bytes);
-
-#define B200_DEFINE_TILE_LANES(T, ALG, L)                                                                              \
-    template <>                                                                                                        \
-    void launch_tile_lanes<T, ALG, L>(const K4Params &kp, bool smem, bool tm, bool et, bool wide, bool idx16, int ctas, int threads, size_t smem_bytes, \
-                                      cudaStream_t s)                                                                  \
-    {                                                                                                                  \
-        constexpr int NB = (ALG == ALG_MS) ? (1024 / B200_TILE_MAX_THREADS) : 1;                                       \
-        typedef uint32_t U32;                                                                                          \
-        typedef uint16_t U16;                                                                                          \
-        if (smem && tm && idx16 && (et || ALG != ALG_MS)) launch_tile_one<T, U16, ALG, true, L, true, true, 1>(kp, ctas, threads, smem_bytes, s); \
-        else if (smem && tm && idx16) launch_tile_one<T, U16, ALG, true, L, true, ALG != ALG_MS, 1>(kp, ctas, threads, smem_bytes, s); \
-        else if (smem && tm && (et || ALG != ALG_MS)) launch_tile_one<T, U32, ALG, true, L, true, true, 1>(kp, ctas, threads, smem_bytes, s); \
-        else if (smem && tm) launch_tile_one<T, U32, ALG, true, L, true, ALG != ALG_MS, 1>(kp, ctas, threads, smem_bytes, s); \
-        else if (smem) launch_tile_one<T, U32, ALG, true, L, false, true, 1>(kp, ctas, threads, smem_bytes, s);        \
-        else if (wide) launch_tile_one<T, U32, ALG, false, L, false, true, 1>(kp, ctas, threads, smem_bytes, s);       \
-        else launch_tile_one<T, U32, ALG, false, L, false, true, NB>(kp, ctas, threads, smem_bytes, s);                \
-    }                                                                                                                  \
-    template <>                                                                                                        \
-    int occupancy_tile_lanes<T, ALG, L>(bool smem, bool tm, bool et, bool wide, bool idx16, int threads, size_t smem_bytes) \
-    {                                                                                                                  \
-        constexpr int NB = (ALG == ALG_MS) ? (1024 / B200_TILE_MAX_THREADS) : 1;                                       \
-        typedef uint32_t U32;                                                                                          \
-        typedef uint16_t U16;                                                                                          \
-        return (smem && tm && idx16 && (et || ALG != ALG_MS)) ? occupancy_tile_one<T, U16, ALG, true, L, true, true, 1>(threads, smem_bytes) \
-               : (smem && tm && idx16) ? occupancy_tile_one<T, U16, ALG, true, L, true, ALG != ALG_MS, 1>(threads, smem_bytes) \
-               : (smem && tm && (et || ALG != ALG_MS)) ? occupancy_tile_one<T, U32, ALG, true, L, true, true, 1>(threads, smem_bytes) \
-               : (smem && tm)     ? occupancy_tile_one<T, U32, ALG, true, L, true, ALG != ALG_MS, 1>(threads, smem_bytes) \
-               : smem             ? occupancy_tile_one<T, U32, ALG, true, L, false, true, 1>(threads, smem_bytes)      \
-               : wide             ? occupancy_tile_one<T, U32, ALG, false, L, false, true, 1>(threads, smem_bytes)     \
-                                  : occupancy_tile_one<T, U32, ALG, false, L, false, true, NB>(threads, smem_bytes);   \
+    const void *tile_variant(bool smem, bool tm, bool et, bool wide, bool idx16)
+    {
+        constexpr int NB = (ALG == ALG_MS) ? (1024 / B200_TILE_MAX_THREADS) : 1;
+        typedef uint32_t U32;
+        typedef uint16_t U16;
+        if (smem && tm && idx16 && (et || ALG != ALG_MS)) return (const void *)tile4_kernel<T, U16, ALG, true, L, true, true, 1>;
+        if (smem && tm && idx16) return (const void *)tile4_kernel<T, U16, ALG, true, L, true, ALG != ALG_MS, 1>;
+        if (smem && tm && (et || ALG != ALG_MS)) return (const void *)tile4_kernel<T, U32, ALG, true, L, true, true, 1>;
+        if (smem && tm) return (const void *)tile4_kernel<T, U32, ALG, true, L, true, ALG != ALG_MS, 1>;
+        if (smem) return (const void *)tile4_kernel<T, U32, ALG, true, L, false, true, 1>;
+        if (wide) return (const void *)tile4_kernel<T, U32, ALG, false, L, false, true, 1>;
+        return (const void *)tile4_kernel<T, U32, ALG, false, L, false, true, NB>;
     }
 
-    template <typename T, int ALG>
-    void launch_tile_family(const K4Params &kp, bool smem, bool tm, bool et, bool wide, bool idx16, int lanes, int ctas, int threads, size_t smem_bytes, cudaStream_t s)
+    extern template const void *tile_variant<double, ALG_BP, 1>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<double, ALG_BP, 2>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<double, ALG_BP, 4>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<double, ALG_MS, 1>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<double, ALG_MS, 2>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<double, ALG_MS, 4>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_BP, 1>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_BP, 2>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_BP, 4>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_MS, 1>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_MS, 2>(bool, bool, bool, bool, bool);
+    extern template const void *tile_variant<float, ALG_MS, 4>(bool, bool, bool, bool, bool);
+
+    // the tile kernel for (precision, algorithm, lanes per node: 1, 2 or 4) and the variant switches
+    inline const void *tile_kernel(bool f32, int alg, int lanes, bool smem, bool tm, bool et, bool wide, bool idx16)
     {
-        switch (lanes)
-        {
-        case 1: launch_tile_lanes<T, ALG, 1>(kp, smem, tm, et, wide, idx16, ctas, threads, smem_bytes, s); return;
-        case 2: launch_tile_lanes<T, ALG, 2>(kp, smem, tm, et, wide, idx16, ctas, threads, smem_bytes, s); return;
-        case 4: launch_tile_lanes<T, ALG, 4>(kp, smem, tm, et, wide, idx16, ctas, threads, smem_bytes, s); return;
-        default: throw std::runtime_error("lanes per node must be 1, 2 or 4");
-        }
-    }
-    template <typename T, int ALG>
-    int tile_family_occupancy(bool smem, bool tm, bool et, bool wide, bool idx16, int lanes, int threads, size_t smem_bytes)
-    {
-        switch (lanes)
-        {
-        case 1: return occupancy_tile_lanes<T, ALG, 1>(smem, tm, et, wide, idx16, threads, smem_bytes);
-        case 2: return occupancy_tile_lanes<T, ALG, 2>(smem, tm, et, wide, idx16, threads, smem_bytes);
-        case 4: return occupancy_tile_lanes<T, ALG, 4>(smem, tm, et, wide, idx16, threads, smem_bytes);
-        default: throw std::runtime_error("lanes per node must be 1, 2 or 4");
-        }
+        typedef const void *(*Variant)(bool, bool, bool, bool, bool);
+        static const Variant variants[2][2][3] = {
+            {{tile_variant<double, ALG_MS, 1>, tile_variant<double, ALG_MS, 2>, tile_variant<double, ALG_MS, 4>},
+             {tile_variant<double, ALG_BP, 1>, tile_variant<double, ALG_BP, 2>, tile_variant<double, ALG_BP, 4>}},
+            {{tile_variant<float, ALG_MS, 1>, tile_variant<float, ALG_MS, 2>, tile_variant<float, ALG_MS, 4>},
+             {tile_variant<float, ALG_BP, 1>, tile_variant<float, ALG_BP, 2>, tile_variant<float, ALG_BP, 4>}}};
+        if (lanes != 1 && lanes != 2 && lanes != 4) throw std::runtime_error("lanes per node must be 1, 2 or 4");
+        return variants[f32][alg == ALG_BP][lanes / 2](smem, tm, et, wide, idx16);
     }
 } // namespace b200

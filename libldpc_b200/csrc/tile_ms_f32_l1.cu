@@ -2,5 +2,5 @@
 #include "tile_launch.cuh"
 namespace b200
 {
-    B200_DEFINE_TILE_LANES(float, ALG_MS, 1)
+    template const void *tile_variant<float, ALG_MS, 1>(bool, bool, bool, bool, bool);
 }
