@@ -255,6 +255,28 @@ typedef struct
 LDPC_B200_API int ldpc_b200_sim_point_log(ldpc_b200_ctx *ctx, decoder_param dp, const char *channel, double x, uint64_t seed,
                             uint32_t point, uint64_t frame0, uint64_t n_frames, uint64_t counters[4],
                             ldpc_b200_error_record *records, int64_t capacity, int64_t *n_errors);
+/* Batched replay of frames in error, on the GPU: for every global frame index frames[i] of sweep point `point` the channel
+ * regenerates the decoder input, the decoder runs under the context's current tuning (precision, residency, schedule,
+ * modulation; the erasure decode mode on "BEC") and the decisions are compared with the transmitted word.  reports[i] describes
+ * frames[i] (same order; repeated and unsorted indices are allowed); its failed bits are failed_bits[bits_offset ..
+ * bits_offset + bit_errors): the variable ids of the transmitted positions whose decision differs, in transmitted order; its
+ * failed checks are failed_checks[checks_offset .. checks_offset + syndrome_weight): the unsatisfied checks of the decisions,
+ * ascending.  syndrome_weight = 0 with bit_errors > 0 is an undetected error (the decoder stopped on another codeword).  With
+ * M-ASK the decoder sees the all-zero word (ldpc_b200_set_modulation), and the decisions are compared with it.
+ * *bits_needed / *checks_needed (may be NULL) receive the total list lengths.  When a capacity is too small the call fails and
+ * writes nothing but those two: call again with capacities of at least that size.  Blocking; HOST buffers. */
+typedef struct
+{
+    uint64_t frame;                      /* global frame index of the sweep point */
+    int32_t iterations;                  /* reference iteration count of the replayed decode */
+    uint32_t bit_errors;                 /* = number of failed_bits of this frame */
+    uint32_t syndrome_weight;            /* = number of failed_checks of this frame */
+    int64_t bits_offset, checks_offset;  /* into failed_bits / failed_checks */
+} ldpc_b200_frame_report;
+LDPC_B200_API int ldpc_b200_error_report(ldpc_b200_ctx *ctx, decoder_param dp, const char *channel, double x, uint64_t seed,
+                                         uint32_t point, const uint64_t *frames, int64_t n_frames, ldpc_b200_frame_report *reports,
+                                         int32_t *failed_bits, int64_t bits_capacity, int32_t *failed_checks, int64_t checks_capacity,
+                                         int64_t *bits_needed, int64_t *checks_needed);
 /* Asynchronous variant: d_counters is a DEVICE array of 5 uint64 that the kernel accumulates into
  * ({frame errors, bit errors, frames, sum of reference iteration counts, sum of executed iterations}). */
 LDPC_B200_API int ldpc_b200_sim_point_async(ldpc_b200_ctx *ctx, decoder_param dp, const char *channel, double x, uint64_t seed,

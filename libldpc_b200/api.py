@@ -46,6 +46,11 @@ class error_record(ct.Structure):  # ldpc_b200_error_record
     _fields_ = [("frame", ct.c_uint64), ("bit_errors", ct.c_uint32), ("iterations", ct.c_int32)]
 
 
+class frame_report(ct.Structure):  # ldpc_b200_frame_report
+    _fields_ = [("frame", ct.c_uint64), ("iterations", ct.c_int32), ("bit_errors", ct.c_uint32), ("syndrome_weight", ct.c_uint32),
+                ("bits_offset", ct.c_int64), ("checks_offset", ct.c_int64)]
+
+
 class stats(ct.Structure):
     _fields_ = [("device_ms", ct.c_double), ("launches", ct.c_uint64), ("frames", ct.c_uint64), ("edge_iterations", ct.c_uint64),
                 ("frames_per_cta", ct.c_int), ("threads_per_cta", ct.c_int), ("ctas", ct.c_int), ("residency", ct.c_int),
@@ -65,7 +70,8 @@ HANDLE_SYMBOLS = ("ldpc_b200_last_error", "ldpc_b200_version", "ldpc_b200_device
                   "ldpc_b200_get_puncture", "ldpc_b200_get_layout", "ldpc_b200_rank", "ldpc_b200_encode", "ldpc_b200_syndrome",
                   "ldpc_b200_decode_batch", "ldpc_b200_decode_batch_device", "ldpc_b200_decode_bec_batch", "ldpc_b200_channel",
                   "ldpc_b200_sim_point", "ldpc_b200_sim_point_async", "ldpc_b200_simulate", "ldpc_b200_simulate_ex", "ldpc_b200_get_stats",
-                  "ldpc_b200_reset_stats", "ldpc_b200_smem_probe", "ldpc_b200_sim_point_log", "ldpc_b200_prepare", "ldpc_b200_decode_batch_ex", "ldpc_b200_decode_batch_device_ex", "ldpc_b200_get_bec_layout", "ldpc_b200_fp64_probe", "ldpc_b200_set_layers", "ldpc_b200_load_layers", "ldpc_b200_get_layers", "ldpc_b200_set_modulation")
+                  "ldpc_b200_reset_stats", "ldpc_b200_smem_probe", "ldpc_b200_sim_point_log", "ldpc_b200_prepare", "ldpc_b200_decode_batch_ex", "ldpc_b200_decode_batch_device_ex", "ldpc_b200_get_bec_layout", "ldpc_b200_fp64_probe", "ldpc_b200_set_layers", "ldpc_b200_load_layers", "ldpc_b200_get_layers", "ldpc_b200_set_modulation",
+                  "ldpc_b200_error_report")
 
 _lib = None
 
@@ -142,6 +148,8 @@ def load_library(path=None):
     L.ldpc_b200_fp64_probe.argtypes = [vp, ct.POINTER(ct.c_double)]
     L.ldpc_b200_sim_point_log.argtypes = [vp, decoder_param, ct.c_char_p, ct.c_double, u64, u32, u64, u64, ct.POINTER(u64), ct.POINTER(error_record),
                                           i64, ct.POINTER(i64)]
+    L.ldpc_b200_error_report.argtypes = [vp, decoder_param, ct.c_char_p, ct.c_double, u64, u32, ct.POINTER(u64), i64, ct.POINTER(frame_report),
+                                         ct.POINTER(ct.c_int32), i64, ct.POINTER(ct.c_int32), i64, ct.POINTER(i64), ct.POINTER(i64)]
     if path is None:
         _lib = L
     return L
@@ -362,6 +370,34 @@ class Context:
         bad = tx[hard[0][tx] != cw[0][tx]]
         return dict(frame=int(frame), iterations=int(its[0]), failed_bits=[int(b) for b in bad], hamming_distance=int(len(bad)),
                     failed_checks=[int(i) for i in np.nonzero(synd)[0]], syndrome_weight=int(synd.sum()))
+
+    def error_reports(self, channel, x, seed, point, frames, decoding="BP", iterations=50, early_term=True):
+        """error_report for many frames at once, on the GPU (ldpc_b200_error_report): one dict per entry of `frames` (global frame
+        indices of sweep point `point`; any order, repeats allowed), with the keys and values of error_report, under the current
+        tuning.  With M-ASK the decisions are compared with the all-zero word the decoder sees."""
+        fr = np.ascontiguousarray(frames, np.uint64).reshape(-1)
+        n = fr.size
+        rep = (frame_report * max(n, 1))()
+        cap = [max(4096, 64 * n)] * 2
+        for attempt in range(2):
+            bits, checks = np.empty(cap[0], np.int32), np.empty(cap[1], np.int32)
+            nb, nk = ct.c_int64(-1), ct.c_int64(-1)
+            rc = self.lib.ldpc_b200_error_report(self._h, self._dp(decoding, iterations, early_term), channel.encode(), float(x), int(seed), int(point),
+                                                 _p(fr, ct.c_uint64), n, rep, _p(bits, ct.c_int32), cap[0], _p(checks, ct.c_int32), cap[1],
+                                                 ct.byref(nb), ct.byref(nk))
+            if rc == 0:
+                break
+            if attempt or nb.value < 0 or (nb.value <= cap[0] and nk.value <= cap[1]):
+                self._check(rc)
+            cap = [nb.value, nk.value]      # the lists did not fit: once more with their exact sizes
+        out = []
+        for i in range(n):
+            r = rep[i]
+            fb = bits[r.bits_offset:r.bits_offset + r.bit_errors].tolist()
+            fc = checks[r.checks_offset:r.checks_offset + r.syndrome_weight].tolist()
+            out.append(dict(frame=int(r.frame), iterations=int(r.iterations), failed_bits=fb, hamming_distance=int(r.bit_errors),
+                            failed_checks=fc, syndrome_weight=int(r.syndrome_weight)))
+        return out
 
     def prepare(self, decoding="BP", iterations=50, early_term=True, nframes=1 << 20):
         """Runs the one-off kernel-shape trial for this (decoder, precision) now, so that asynchronous launches use its outcome."""

@@ -15,7 +15,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-ccbin", "/usr/bin/g++", "-Xcompiler", "-fPIC,-Wall,-Wno-unused-function,-fvisibility=hidden"]
 TILE_SOURCES = ["tile_%s_%s_l%d.cu" % (a, t, l) for a in ("bp", "ms") for t in ("f64", "f32") for l in (1, 2, 4)]  # slowest first
 SOURCES = TILE_SOURCES + ["layered.cu", "engine.cu", "code.cpp", "sim_driver.cpp", "shim.cpp"]
-HEADERS = ["exports.map", "engine.hpp", "code.hpp", "kernels.cuh", "tile4.cuh", "tile_launch.cuh", "bec_kernel.cuh", "bec_slice.cuh", "layered.cuh", "../../include/ldpc_b200.h"]
+HEADERS = ["exports.map", "engine.hpp", "code.hpp", "kernels.cuh", "tile4.cuh", "tile_launch.cuh", "bec_kernel.cuh", "bec_slice.cuh", "layered.cuh", "report.cuh", "../../include/ldpc_b200.h"]
 OBJDIR = os.path.join(HERE, "build")
 if os.environ.get("B200_PHASE_TIMING"):  # debug: per-warp phase cycle counts printed by CTA 0
     COMMON = COMMON + ["-DB200_PHASE_TIMING=1"]

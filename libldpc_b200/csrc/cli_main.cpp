@@ -6,7 +6,8 @@
 // Negative MIN/MAX are positionals, as with the reference's argument parser.
 // B200 extras (do not exist in the reference): --precision f64|f32, --device N, --gpus N / --devices LIST (frames of every
 // round sharded over N GPUs of this process, one host thread per shard; the counters are summed on the host, results do not
-// depend on the number of shards).
+// depend on the number of shards), --error-log FILE (per sweep point, the first --frame-error-count frames in error, replayed on the
+// GPU: failed bits and checks; see the usage text).
 // The CLI is a client of the C ABI only (include/ldpc_b200.h): the library exports nothing else.
 #include <algorithm>
 #include <cstdio>
@@ -14,6 +15,7 @@
 #include <array>
 #include <cstring>
 #include <iostream>
+#include <map>
 #include <stdexcept>
 #include <memory>
 #include <string>
@@ -49,7 +51,10 @@ namespace
         "--ms-scale          \tB200 only: with --schedule layered and BP_MS: normalisation factor of the check outputs in 1/64 steps (Default: 1 = plain min-sum)\n"
         "--modulation        \tB200 only: M-ASK with bit-metric decoding on the AWGN channel, M = 4, 8, ... (Gray labels, consecutive bit mapper; Default: 2 = BPSK)\n"
         "--layers            \tB200 only: layer file for --schedule layered (legacy format: nl: N / cn[i]: W / W check indices); default: built-in layering\n"
-        "--devices           \tB200 only: explicit device list for the shards, e.g. 0,1,2,3 (an index may repeat: several shards on one GPU)\n";
+        "--devices           \tB200 only: explicit device list for the shards, e.g. 0,1,2,3 (an index may repeat: several shards on one GPU)\n"
+        "--error-log         \tB200 only: file of the frames in error: per point the first --frame-error-count of them in frame order, one line\n"
+        "                    \teach: snr frame iterations bit_errors syndrome_weight failed_bits failed_checks (comma-separated lists, - = empty;\n"
+        "                    \tsyndrome_weight 0 with bit_errors > 0 is an undetected error); written after every round\n";
 
     bool looks_numeric(const std::string &s)
     {
@@ -68,7 +73,16 @@ namespace
         decoder_param dp;
         std::string channel;
         uint64_t seed = 0;
-        ~MultiGpu() { for (auto *c : ctxs) ldpc_b200_close(c); }
+        // --error-log
+        FILE *log = nullptr;
+        uint64_t log_budget = 0;              // frames logged per point (--frame-error-count)
+        std::map<uint32_t, uint64_t> logged;  // point -> frames logged so far
+        uint64_t mismatches = 0;              // logged frames whose replay differs from the sweep's record
+        ~MultiGpu()
+        {
+            for (auto *c : ctxs) ldpc_b200_close(c);
+            if (log) fclose(log);
+        }
     };
     int multi_gpu_round(uint32_t point, double x, uint64_t frame0, uint64_t n, uint64_t *counters, void *user)
     {
@@ -90,6 +104,93 @@ namespace
         {
             if (!err[i].empty()) { std::cout << "Error: GPU " << i << ": " << err[i] << std::endl; return 1; }
             for (int k = 0; k < 4; ++k) counters[k] += part[i][k];
+        }
+        return 0;
+    }
+
+    void write_list(FILE *f, const int32_t *v, uint32_t n)
+    {
+        if (n == 0) fputs("-", f);
+        for (uint32_t i = 0; i < n; ++i) fprintf(f, i ? ",%d" : "%d", (int)v[i]);
+    }
+
+    // A round with the error log.  Every shard records its frames in error (a slice whose errors overflow the record buffer is
+    // run again with room for all of them: the counters are deterministic); the records are merged in global frame order and
+    // the first ones, up to what is left of the point's budget, are replayed on the first context and appended to the log.  The
+    // logged set therefore depends only on (seed, point, frames decoded), not on the shards or the round split.
+    int logged_round(uint32_t point, double x, uint64_t frame0, uint64_t n, uint64_t *counters, void *user)
+    {
+        MultiGpu &m = *static_cast<MultiGpu *>(user);
+        const size_t g = m.ctxs.size();
+        std::vector<std::array<uint64_t, 4>> part(g, std::array<uint64_t, 4>{0, 0, 0, 0});
+        std::vector<std::vector<ldpc_b200_error_record>> recs(g);
+        std::vector<std::string> err(g);
+        std::vector<std::thread> th;
+        for (size_t i = 0; i < g; ++i)
+            th.emplace_back([&, i] {
+                const uint64_t lo = frame0 + n * i / g, hi = frame0 + n * (i + 1) / g;
+                if (hi == lo) return;
+                int64_t cap = 256, n_err = 0;
+                for (;;)
+                {
+                    part[i] = {0, 0, 0, 0};
+                    recs[i].resize((size_t)cap);
+                    if (ldpc_b200_sim_point_log(m.ctxs[i], m.dp, m.channel.c_str(), x, m.seed, point, lo, hi - lo, part[i].data(), recs[i].data(), cap,
+                                                &n_err) != 0)
+                    {
+                        err[i] = ldpc_b200_last_error();
+                        return;
+                    }
+                    if (n_err <= cap) break;
+                    cap = n_err;
+                }
+                recs[i].resize((size_t)n_err);
+            });
+        for (auto &t : th) t.join();
+        std::vector<ldpc_b200_error_record> all;
+        for (size_t i = 0; i < g; ++i)
+        {
+            if (!err[i].empty()) { std::cout << "Error: GPU " << i << ": " << err[i] << std::endl; return 1; }
+            for (int k = 0; k < 4; ++k) counters[k] += part[i][k];
+            all.insert(all.end(), recs[i].begin(), recs[i].end());
+        }
+        std::sort(all.begin(), all.end(), [](const ldpc_b200_error_record &a, const ldpc_b200_error_record &b) { return a.frame < b.frame; });
+        uint64_t &logged = m.logged[point];
+        all.resize((size_t)std::min<uint64_t>(all.size(), m.log_budget > logged ? m.log_budget - logged : 0));
+        if (all.empty()) return 0;
+        std::vector<uint64_t> frames(all.size());
+        for (size_t j = 0; j < all.size(); ++j) frames[j] = all[j].frame;
+        std::vector<ldpc_b200_frame_report> rep(all.size());
+        std::vector<int32_t> bits(4096), checks(4096);
+        for (int attempt = 0;; ++attempt)
+        {
+            int64_t nb = 0, nk = 0;
+            if (ldpc_b200_error_report(m.ctxs[0], m.dp, m.channel.c_str(), x, m.seed, point, frames.data(), (int64_t)frames.size(), rep.data(),
+                                       bits.data(), (int64_t)bits.size(), checks.data(), (int64_t)checks.size(), &nb, &nk) == 0)
+                break;
+            if (attempt > 0 || (nb <= (int64_t)bits.size() && nk <= (int64_t)checks.size()))
+            {
+                std::cout << "Error: error log: " << ldpc_b200_last_error() << std::endl;
+                return 1;
+            }
+            bits.resize((size_t)std::max<int64_t>(nb, 1));
+            checks.resize((size_t)std::max<int64_t>(nk, 1));
+        }
+        for (size_t j = 0; j < rep.size(); ++j)
+        {
+            const ldpc_b200_frame_report &r = rep[j];
+            if (r.iterations != all[j].iterations || r.bit_errors != all[j].bit_errors) ++m.mismatches;
+            fprintf(m.log, "%lf %llu %d %u %u ", x, (unsigned long long)r.frame, (int)r.iterations, (unsigned)r.bit_errors, (unsigned)r.syndrome_weight);
+            write_list(m.log, bits.data() + r.bits_offset, r.bit_errors);
+            fputs(" ", m.log);
+            write_list(m.log, checks.data() + r.checks_offset, r.syndrome_weight);
+            fputs("\n", m.log);
+        }
+        logged += rep.size();
+        if (fflush(m.log) != 0 || ferror(m.log))
+        {
+            std::cout << "Error: error log: write failed" << std::endl;
+            return 1;
         }
         return 0;
     }
@@ -126,7 +227,7 @@ int main(int argc, char **argv)
     unsigned long seed = 0, max_frames = (unsigned long)10e9, fec = 50;
     bool early_term = true;
     int device = 0, gpus = 1;
-    std::string device_list, schedule = "flooding", layer_file;
+    std::string device_list, schedule = "flooding", layer_file, error_log;
     double ms_scale = 1.0;
     int modulation = 2;
     std::vector<std::string> pos;
@@ -159,6 +260,7 @@ int main(int argc, char **argv)
             else if (a == "--layers") layer_file = value();
             else if (a == "--ms-scale") ms_scale = std::stod(value());
             else if (a == "--modulation") modulation = std::stoi(value());
+            else if (a == "--error-log") error_log = value();
             else if (a.size() > 1 && a[0] == '-' && !looks_numeric(a)) throw std::runtime_error("Unknown argument: " + a);
             else pos.push_back(a);
         }
@@ -178,6 +280,18 @@ int main(int argc, char **argv)
             for (int g = 0; g < gpus; ++g) devices.push_back(device + g);
         }
         MultiGpu m;
+        if (!error_log.empty())
+        { // truncated now: a file that cannot be written fails before any work
+            m.log = fopen(error_log.c_str(), "w");
+            if (!m.log)
+            {
+                std::cout << "Error: --error-log: cannot open " << error_log << " for writing" << std::endl;
+                return EXIT_FAILURE;
+            }
+            fputs("snr frame iterations bit_errors syndrome_weight failed_bits failed_checks\n", m.log);
+            fflush(m.log);
+            m.log_budget = fec;
+        }
         ldpc_b200_ctx *ctx = ldpc_b200_open(pos[0].c_str(), gen.c_str(), devices[0]);
         if (!ctx)
         {
@@ -236,9 +350,9 @@ int main(int argc, char **argv)
         std::cout << bar << std::endl;
         bool stop = false;
         int rc;
-        if (devices.size() == 1) rc = ldpc_b200_simulate(ctx, dp, cp, sp, nullptr, &stop, 0, 1, nullptr, nullptr, 0);
+        if (devices.size() == 1 && !m.log) rc = ldpc_b200_simulate(ctx, dp, cp, sp, nullptr, &stop, 0, 1, nullptr, nullptr, 0);
         else
-        {
+        { // the logged sweep takes the round callback on any number of devices
             m.dp = dp; m.channel = channel; m.seed = seed;
             for (size_t g = 1; g < devices.size(); ++g)
             {
@@ -249,14 +363,23 @@ int main(int argc, char **argv)
                 if (modulation != 2) ldpc_b200_set_modulation(c, modulation, nullptr, nullptr);
                 m.ctxs.push_back(c);
             }
-            std::cout << "GPUs: " << devices.size() << " shards on devices ";
-            print_list(std::cout, devices);
-            std::cout << std::endl;
-            rc = ldpc_b200_simulate_ex(ctx, dp, cp, sp, nullptr, &stop, 0, 1, nullptr, multi_gpu_round, &m, 0);
+            if (devices.size() > 1)
+            {
+                std::cout << "GPUs: " << devices.size() << " shards on devices ";
+                print_list(std::cout, devices);
+                std::cout << std::endl;
+            }
+            rc = ldpc_b200_simulate_ex(ctx, dp, cp, sp, nullptr, &stop, 0, 1, nullptr, m.log ? logged_round : multi_gpu_round, &m, 0);
         }
         if (rc != 0)
         {
             std::cout << "Error: ldpc_sim::ldpc_sim() " << ldpc_b200_last_error() << std::endl; // src/sim/ldpcsim.cpp:77-81
+            return EXIT_FAILURE;
+        }
+        if (m.mismatches)
+        {
+            std::cout << "Warning: " << m.mismatches << " frame(s) of the error log replayed with other iteration or bit-error counts than the "
+                      << "sweep recorded: their lines do not describe the failure" << std::endl;
             return EXIT_FAILURE;
         }
     }

@@ -14,6 +14,7 @@
 #include "bec_kernel.cuh"
 #include "bec_slice.cuh"
 #include "layered.cuh"
+#include "report.cuh"
 
 namespace b200
 {
@@ -1380,13 +1381,16 @@ namespace b200
         CUDA_OK(cudaStreamSynchronize(s));
     }
 
-    // Stand-alone channel kernel: the same generator code as the fused path, one thread per Philox block.
+    // Stand-alone channel kernel: the same generator code as the fused path, one thread per Philox block.  Output row fr holds
+    // global frame frame0 + fr, or with GATHER frames[fr] (the replay of a list of logged frames).
+    template <bool GATHER>
     __global__ void channel_kernel(int kind, int nc, int nct, const int32_t *__restrict__ bit_pos, const int32_t *__restrict__ punct, int n_punct,
                                    const int32_t *__restrict__ shorten, int n_short, double sigma, double llr_scale, double delta, uint32_t thr,
                                    uint64_t seed, uint32_t point, uint64_t frame0, int64_t n_frames, uint8_t *cw, double *llr, uint8_t *llr_u8,
                                    const int32_t *__restrict__ g_col_ptr, const int32_t *__restrict__ g_row, int g_rows, int g_cols, AskParams ask,
-                                   double sigma2)
+                                   double sigma2, const uint64_t *__restrict__ frames)
     {
+        auto frame_of = [&](int64_t fr) -> uint64_t { return GATHER ? frames[fr] : frame0 + fr; };
         if (kind == SRC_ASK)
         { // M-ASK with bit-metric decoding: one thread per Philox block of four symbols (same arithmetic as tile4.cuh frame_pass)
             const int nsblk = (ask.n_sym + 3) / 4;
@@ -1396,13 +1400,13 @@ namespace b200
                 const int64_t fr = g / nsblk;
                 const int q = (int)(g % nsblk);
                 const size_t base = (size_t)fr * nc;
-                const u32x4 r = channel_block(seed, point, 0, frame0 + fr, (uint32_t)q);
+                const u32x4 r = channel_block(seed, point, 0, frame_of(fr), (uint32_t)q);
                 float z[4];
                 normal_pair(r.x, r.y, z[0], z[1]);
                 normal_pair(r.z, r.w, z[2], z[3]);
                 for (int k = 0; k < 4; ++k)
                     if (q + k * nsblk < ask.n_sym)
-                        ask_symbol(ask, seed, point, frame0 + fr, q + k * nsblk, z[k], sigma, sigma2, [&](int v, double l, uint32_t c) {
+                        ask_symbol(ask, seed, point, frame_of(fr), q + k * nsblk, z[k], sigma, sigma2, [&](int v, double l, uint32_t c) {
                             llr[base + v] = l;
                             if (cw) cw[base + v] = (uint8_t)c;
                         });
@@ -1423,7 +1427,7 @@ namespace b200
             for (int q = g_col_ptr[v]; q < g_col_ptr[v + 1]; ++q)
             {
                 const int r = g_row[q];
-                const u32x4 w = channel_block(seed, point, 1, frame0 + fr, (uint32_t)r >> 7);
+                const u32x4 w = channel_block(seed, point, 1, frame_of(fr), (uint32_t)r >> 7);
                 const uint32_t q4[4] = {w.x, w.y, w.z, w.w};
                 b ^= q4[(r >> 5) & 3] >> (r & 31);
             }
@@ -1435,7 +1439,7 @@ namespace b200
         {
             const int64_t fr = g / nblk;
             const int j = (int)(g % nblk);
-            const u32x4 r = channel_block(seed, point, 0, frame0 + fr, (uint32_t)j);
+            const u32x4 r = channel_block(seed, point, 0, frame_of(fr), (uint32_t)j);
             const size_t base = (size_t)fr * nc;
             if (kind == SRC_AWGN)
             { // the same arithmetic as the fused path (tile4.cuh frame_pass)
@@ -1495,14 +1499,28 @@ namespace b200
         }
     }
 
+    // Enqueues the channel kernel on s: rows of global frames frame0 + fr, or frames[fr] when `frames` (device) is given.
+    // kind = SRC_AWGN is M-ASK under the current modulation.
+    void Engine::launch_channel(int kind, double x, uint64_t seed, uint32_t point, uint64_t frame0, const uint64_t *frames, int64_t n,
+                                uint8_t *d_cw, double *d_llr, uint8_t *d_u8, cudaStream_t s)
+    {
+        AskParams ask{};
+        if (kind == SRC_AWGN && ask_M > 2) { kind = SRC_ASK; ask_fill(&ask); }
+        const ChannelConsts cc = channel_consts(kind, x);
+        const int g_rows = (has_gen && !tuning.zero_codeword) ? G.mc : 0, g_cols = has_gen ? G.nc : 0;
+        auto fn = frames ? channel_kernel<true> : channel_kernel<false>;
+        fn<<<sm_count_ * 4, 256, 0, s>>>(kind, H.nc, H.nct(), d_bit_pos_.get(), d_punct_.get(), (int)H.puncture.size(), d_short_.get(),
+                                         (int)H.shorten.size(), cc.sigma, cc.llr_scale, cc.delta, cc.thr, seed, point, frame0, n, d_cw, d_llr, d_u8,
+                                         d_g_col_ptr_.get(), d_g_row_.get(), g_rows, g_cols, ask, cc.sigma2, frames);
+        CUDA_OK(cudaGetLastError());
+    }
+
     void Engine::channel_host(const std::string &channel, double x, uint64_t seed, uint32_t point, uint64_t frame0, int64_t n,
                               uint8_t *cw, double *llr, uint8_t *llr_u8)
     {
         if (n <= 0) return;
         ensure_cuda();
-        int kind = channel_kind(channel);
-        AskParams ask{};
-        if (kind == SRC_AWGN && ask_M > 2) { kind = SRC_ASK; ask_fill(&ask); }
+        const int kind = channel_kind(channel);
         cudaStream_t s = stream_.get();
         const size_t nc = H.nc;
         DevPtr<double> d_llr;
@@ -1510,16 +1528,106 @@ namespace b200
         if (kind == SRC_BEC) { if (!llr_u8) throw std::runtime_error("llr_u8 buffer required for BEC"); d_u8 = device_alloc<uint8_t>(n * nc); }
         else { if (!llr) throw std::runtime_error("llr buffer required"); d_llr = device_alloc<double>(n * nc); }
         if (cw) d_cw = device_alloc<uint8_t>(n * nc);
-        const ChannelConsts cc = channel_consts(kind, x);
-        channel_kernel<<<sm_count_ * 4, 256, 0, s>>>(kind, (int)nc, H.nct(), d_bit_pos_.get(), d_punct_.get(), (int)H.puncture.size(), d_short_.get(),
-                                                     (int)H.shorten.size(), cc.sigma, cc.llr_scale, cc.delta, cc.thr, seed, point, frame0, n, d_cw.get(),
-                                                     d_llr.get(), d_u8.get(), d_g_col_ptr_.get(), d_g_row_.get(), (has_gen && !tuning.zero_codeword) ? G.mc : 0,
-                                                     has_gen ? G.nc : 0, ask, cc.sigma2);
-        CUDA_OK(cudaGetLastError());
+        launch_channel(kind, x, seed, point, frame0, nullptr, n, d_cw.get(), d_llr.get(), d_u8.get(), s);
         if (d_llr) CUDA_OK(cudaMemcpyAsync(llr, d_llr.get(), n * nc * sizeof(double), cudaMemcpyDeviceToHost, s));
         if (d_u8) CUDA_OK(cudaMemcpyAsync(llr_u8, d_u8.get(), n * nc, cudaMemcpyDeviceToHost, s));
         if (d_cw) CUDA_OK(cudaMemcpyAsync(cw, d_cw.get(), n * nc, cudaMemcpyDeviceToHost, s));
         CUDA_OK(cudaStreamSynchronize(s));
+    }
+
+    // Replay of logged frames: the gather channel regenerates their decoder inputs, the decode runs under the current tuning
+    // (the erasure decode mode on the BEC, as decode_bec_host), and report_kernel compares the decisions with the transmitted
+    // word.  Chunks of about 32 MB of decoder input, whole waves of the persistent grid.
+    void Engine::error_report(const decoder_param &dp, const std::string &channel, double x, uint64_t seed, uint32_t point, const uint64_t *frames,
+                              int64_t n, ldpc_b200_frame_report *reports, std::vector<int32_t> &bits, std::vector<int32_t> &checks)
+    {
+        const int kind = channel_kind(channel);
+        if (n < 0 || (n > 0 && (!frames || !reports))) throw std::runtime_error("error_report: bad frame list");
+        bits.clear();
+        checks.clear();
+        if (n == 0) return;
+        ensure_cuda();
+        cudaStream_t s = stream_.get();
+        const bool bec = kind == SRC_BEC, ask = kind == SRC_AWGN && ask_M > 2;
+        const size_t nc = H.nc;
+        if (!d_chk_var_)
+        {
+            std::vector<int32_t> ptr(H.row_ptr.begin(), H.row_ptr.end()), var(H.nnz);
+            for (int q = 0; q < H.nnz; ++q) var[q] = (int32_t)H.e_col[H.row_edge[q]];
+            d_chk_ptr_ = upload(ptr);
+            d_chk_var_ = upload(var);
+        }
+        int64_t chunk = std::max<int64_t>((int64_t)((32ull << 20) / (nc * (bec ? 1 : sizeof(double)))), 1);
+        if (!bec)
+        {
+            maybe_autotune(alg_of(dp), dp, (uint64_t)n, s);
+            const Config c = choose(tuning.precision, alg_of(dp), ~0ull >> 1);
+            const int64_t wave = (int64_t)c.ctas * c.fpc;
+            chunk = std::max<int64_t>(wave, chunk / wave * wave);
+        }
+        chunk = std::min<int64_t>(chunk, n);
+        const DevPtr<uint64_t> d_frames = device_alloc<uint64_t>(chunk);
+        const DevPtr<uint8_t> d_cw = device_alloc<uint8_t>(chunk * nc), d_hard = device_alloc<uint8_t>(chunk * nc);
+        DevPtr<uint8_t> d_u8;
+        DevPtr<double> d_llr;
+        if (bec) d_u8 = device_alloc<uint8_t>(chunk * nc);
+        else d_llr = device_alloc<double>(chunk * nc);
+        const DevPtr<int32_t> d_iters = device_alloc<int32_t>(chunk);
+        const DevPtr<uint32_t> d_counts = device_alloc<uint32_t>(2 * chunk);
+        const DevPtr<int64_t> d_offsets = device_alloc<int64_t>(2 * chunk);
+        DevBuf d_bits, d_checks;
+        std::vector<int32_t> iters(chunk);
+        std::vector<uint32_t> counts(2 * chunk);
+        std::vector<int64_t> offsets(2 * chunk);
+        ReportParams rp{};
+        rp.hard = d_hard.get(); rp.cw = ask ? nullptr : d_cw.get(); // M-ASK: the decoder sees the all-zero word (set_modulation)
+        rp.bit_pos = d_bit_pos_.get(); rp.chk_ptr = d_chk_ptr_.get(); rp.chk_var = d_chk_var_.get();
+        rp.nc = H.nc; rp.nct = H.nct(); rp.mc = H.mc;
+        rp.counts = d_counts.get(); rp.offsets = d_offsets.get();
+        for (int64_t o = 0; o < n; o += chunk)
+        {
+            const int64_t m = std::min(chunk, n - o);
+            CUDA_OK(cudaMemcpyAsync(d_frames.get(), frames + o, m * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+            launch_channel(kind, x, seed, point, 0, d_frames.get(), m, ask ? nullptr : d_cw.get(), d_llr.get(), d_u8.get(), s);
+            FrameSource src;
+            src.kind = SRC_LLR;
+            if (bec) { src.d_bec_in = d_u8.get(); src.d_bec_cw = d_cw.get(); }
+            else src.d_llr = d_llr.get();
+            FrameSink sink;
+            sink.d_hard = d_hard.get(); sink.d_iters = d_iters.get();
+            launch(dp, src, sink, (uint64_t)m, s);
+            rp.n = m;
+            const int blocks = clamp_grid(sm_count_ * 8, (uint64_t)(m + 7) / 8); // 8 warps (frames) per block
+            report_kernel<false><<<blocks, 256, 0, s>>>(rp);
+            CUDA_OK(cudaGetLastError());
+            CUDA_OK(cudaMemcpyAsync(counts.data(), d_counts.get(), 2 * m * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+            CUDA_OK(cudaMemcpyAsync(iters.data(), d_iters.get(), m * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+            CUDA_OK(cudaStreamSynchronize(s));
+            int64_t nb = 0, nk = 0;
+            for (int64_t i = 0; i < m; ++i)
+            {
+                offsets[2 * i] = nb; offsets[2 * i + 1] = nk;
+                ldpc_b200_frame_report &r = reports[o + i];
+                r.frame = frames[o + i]; r.iterations = iters[i];
+                r.bit_errors = counts[2 * i]; r.syndrome_weight = counts[2 * i + 1];
+                r.bits_offset = (int64_t)bits.size() + nb; r.checks_offset = (int64_t)checks.size() + nk;
+                nb += counts[2 * i];
+                nk += counts[2 * i + 1];
+            }
+            if (nb + nk == 0) continue;
+            grow(d_bits, std::max<int64_t>(nb, 1) * sizeof(int32_t));
+            grow(d_checks, std::max<int64_t>(nk, 1) * sizeof(int32_t));
+            rp.failed_bits = (int32_t *)d_bits.p.get(); rp.failed_checks = (int32_t *)d_checks.p.get();
+            CUDA_OK(cudaMemcpyAsync(d_offsets.get(), offsets.data(), 2 * m * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+            report_kernel<true><<<blocks, 256, 0, s>>>(rp);
+            CUDA_OK(cudaGetLastError());
+            const size_t b0 = bits.size(), k0 = checks.size();
+            bits.resize(b0 + nb);
+            checks.resize(k0 + nk);
+            if (nb) CUDA_OK(cudaMemcpyAsync(bits.data() + b0, d_bits.p.get(), nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+            if (nk) CUDA_OK(cudaMemcpyAsync(checks.data() + k0, d_checks.p.get(), nk * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+            CUDA_OK(cudaStreamSynchronize(s));
+        }
     }
 } // namespace b200
 

@@ -99,6 +99,11 @@ namespace b200
                        uint64_t frame0, uint64_t n_frames, uint64_t counters[5], float *device_ms);
         void sim_point_log(const decoder_param &dp, const std::string &channel, double x, uint64_t seed, uint32_t point, uint64_t frame0,
                            uint64_t n_frames, uint64_t counters[5], ldpc_b200_error_record *records, int64_t capacity, int64_t *n_errors);
+        // Replays global frames frames[0 .. n) of a sweep point (any order, repeats allowed) under the current tuning and
+        // reports each: reports[i] with offsets into `bits` (failed transmitted positions, in transmitted order) and `checks`
+        // (unsatisfied checks, ascending), which are replaced.  Blocking.
+        void error_report(const decoder_param &dp, const std::string &channel, double x, uint64_t seed, uint32_t point, const uint64_t *frames,
+                          int64_t n, ldpc_b200_frame_report *reports, std::vector<int32_t> &bits, std::vector<int32_t> &checks);
         void sim_point_async(const decoder_param &dp, const std::string &channel, double x, uint64_t seed, uint32_t point,
                              uint64_t frame0, uint64_t n_frames, unsigned long long *d_counters, void *stream, bool may_block = false);
 
@@ -166,6 +171,8 @@ namespace b200
         void release_state(CUstream_st *s);
         bool try_seg_layout(int lanes, int threads, int isz);
         static int channel_kind(const std::string &name);
+        void launch_channel(int kind, double x, uint64_t seed, uint32_t point, uint64_t frame0, const uint64_t *frames, int64_t n,
+                            uint8_t *d_cw, double *d_llr, uint8_t *d_u8, CUstream_st *s);
         const void *tile_fn(const Config &c, bool et); // the tile kernel of c (early termination: et), its attributes set
         // dynamic shared-memory opt-in (max_shared: and the all-shared carveout) of a kernel, set on this engine's first use of it
         void set_smem_attributes(const void *fn, int smem_optin, bool max_shared);
@@ -204,6 +211,7 @@ namespace b200
         Event ev_state_; // recorded after every launch that uses the state block
         DevPtr<int32_t> d_bit_pos_, d_punct_, d_short_;
         DevPtr<int32_t> d_g_col_ptr_, d_g_row_; // generator matrix by column (device)
+        DevPtr<int32_t> d_chk_ptr_, d_chk_var_; // check-major CSR of H: variable ids (error_report)
         DevPtr<int32_t> d_bs_row_ptr_, d_bs_col_ptr_; // bit-sliced BEC kernel
         DevPtr<uint16_t> d_bs_row_slot_, d_bs_col_slot_;
         DevPtr<uint8_t> d_bs_tx_flag_;

@@ -1,5 +1,6 @@
 // C-ABI shim: the six reference symbols (src/shared.cpp:9-78) over a process-global context, plus
 // the handle-based ldpc_b200_* API (include/ldpc_b200.h).  No exceptions cross this boundary.
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -18,6 +19,7 @@ static_assert(sizeof(channel_param) == 40 && offsetof(channel_param, xRange) == 
 static_assert(sizeof(simulation_param) == 32 && offsetof(simulation_param, maxFrames) == 8 && offsetof(simulation_param, fec) == 16 &&
                   offsetof(simulation_param, resultFile) == 24, "simulation_param layout");
 static_assert(sizeof(sim_results_t) == 48, "sim_results_t layout (src/sim/ldpcsim.h:23-31)");
+static_assert(sizeof(ldpc_b200_frame_report) == 40 && offsetof(ldpc_b200_frame_report, bits_offset) == 24, "ldpc_b200_frame_report layout");
 
 struct ldpc_b200_ctx
 {
@@ -428,6 +430,31 @@ extern "C"
             uint64_t c[5] = {0, 0, 0, 0, 0};
             ctx->eng->sim_point_log(dp, channel, x, seed, point, frame0, n_frames, c, records, capacity, n_errors);
             for (int i = 0; i < 4; ++i) counters[i] += c[i];
+        });
+    }
+
+    int ldpc_b200_error_report(ldpc_b200_ctx *ctx, decoder_param dp, const char *channel, double x, uint64_t seed, uint32_t point,
+                               const uint64_t *frames, int64_t n_frames, ldpc_b200_frame_report *reports, int32_t *failed_bits,
+                               int64_t bits_capacity, int32_t *failed_checks, int64_t checks_capacity, int64_t *bits_needed,
+                               int64_t *checks_needed)
+    {
+        return guarded([&] {
+            if (!ctx || !channel) throw std::runtime_error("null argument");
+            if (n_frames < 0 || bits_capacity < 0 || checks_capacity < 0) throw std::runtime_error("error_report: negative size");
+            if ((n_frames > 0 && (!frames || !reports)) || (bits_capacity > 0 && !failed_bits) || (checks_capacity > 0 && !failed_checks))
+                throw std::runtime_error("null argument");
+            std::vector<ldpc_b200_frame_report> rep((size_t)n_frames);
+            std::vector<int32_t> bits, checks;
+            ctx->eng->error_report(dp, channel, x, seed, point, frames, n_frames, rep.data(), bits, checks);
+            const int64_t nb = (int64_t)bits.size(), nk = (int64_t)checks.size();
+            if (bits_needed) *bits_needed = nb;
+            if (checks_needed) *checks_needed = nk;
+            if (nb > bits_capacity || nk > checks_capacity)
+                throw std::runtime_error("error_report: the reports need " + std::to_string(nb) + " failed bits and " + std::to_string(nk) +
+                                         " failed checks; capacities " + std::to_string(bits_capacity) + " and " + std::to_string(checks_capacity));
+            std::copy(rep.begin(), rep.end(), reports);
+            std::copy(bits.begin(), bits.end(), failed_bits);
+            std::copy(checks.begin(), checks.end(), failed_checks);
         });
     }
 
