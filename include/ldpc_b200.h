@@ -48,7 +48,8 @@ typedef struct
 {
     uint64_t seed;
     double xRange[3]; /* MIN MAX STEP, half-open sweep (src/sim/ldpcsim.cpp:104-110) */
-    const char *type; /* "AWGN" | "BSC" | "BEC" */
+    const char *type; /* "AWGN" | "BSC" | "BEC" | "RAYLEIGH" (B200 extension: x = average SNR in dB; coherence length of the
+                         context, ldpc_b200_set_fading, default 1) */
 } channel_param;
 
 /* reference: src/core/functions.h:121-127 (32 bytes) */
@@ -178,6 +179,13 @@ LDPC_B200_API int ldpc_b200_get_layers(ldpc_b200_ctx *ctx, int *layer_of /*[mc]*
  * ldpc_b200_channel / _sim_point* / _simulate*; flooding schedule. */
 LDPC_B200_API int ldpc_b200_set_modulation(ldpc_b200_ctx *ctx, int M, const int *labels, const int *bit_mapper);
 
+/* Coherence length of the "RAYLEIGH" channel (not in the reference): BPSK over flat Rayleigh fading with perfect channel state
+ * information at the receiver.  Transmitted index t uses fading coefficient floor(t / coherence) of its frame; coherence = 1 (the
+ * default) is fast fading, 0 is one coefficient per frame (quasi-static).  Coefficient c is h = sqrt((a^2 + b^2) / 2) of the first
+ * normal pair of Philox block c of stream 3, E[h^2] = 1; y = sigma z + h (1 - 2 cw) with the AWGN channel's noise z at average
+ * SNR x dB, LLR = y h 2 / sigma^2 (DESIGN.md 3.2).  Per context; negative values fail.  RAYLEIGH with M-ASK (M > 2) fails. */
+LDPC_B200_API int ldpc_b200_set_fading(ldpc_b200_ctx *ctx, int coherence);
+
 /* host-side views of the loaded code (file order; sizes from ldpc_b200_info) */
 LDPC_B200_API int ldpc_b200_get_edges(const ldpc_b200_ctx *ctx, int *rows /*[nnz]*/, int *cols /*[nnz]*/);
 LDPC_B200_API int ldpc_b200_get_bit_pos(const ldpc_b200_ctx *ctx, int *bit_pos /*[nct]*/);
@@ -230,12 +238,12 @@ LDPC_B200_API int ldpc_b200_decode_bec_batch(ldpc_b200_ctx *ctx, decoder_param d
 
 /* Philox channel only: writes the decoder inputs the simulator would generate for global frames
  * [frame0, frame0+n) of sweep point `point`: cw[n][nc] (may be NULL), and llr[n][nc] doubles
- * (AWGN/BSC) or llr_u8[n][nc] (BEC).  HOST buffers. */
+ * (AWGN/BSC/RAYLEIGH) or llr_u8[n][nc] (BEC).  HOST buffers. */
 LDPC_B200_API int ldpc_b200_channel(ldpc_b200_ctx *ctx, const char *channel, double x, uint64_t seed, uint32_t point,
                       uint64_t frame0, int64_t n_frames, uint8_t *cw, double *llr, uint8_t *llr_u8);
 
 /* One Monte-Carlo round of one sweep point, fully on the GPU (channel -> decode -> accounting):
- * global frames [frame0, frame0+n_frames).  counters[4] += {frame errors, bit errors, frames,
+ * global frames [frame0, frame0+n_frames) of channel "AWGN", "BSC", "BEC" or "RAYLEIGH".  counters[4] += {frame errors, bit errors, frames,
  * sum of reference iteration counts} (src/sim/ldpcsim.cpp:175-190).  Blocking; counters on the host.
  * device_ms (may be NULL) receives the CUDA-event time of the kernel(s). */
 LDPC_B200_API int ldpc_b200_sim_point(ldpc_b200_ctx *ctx, decoder_param dp, const char *channel, double x, uint64_t seed,
@@ -245,7 +253,7 @@ LDPC_B200_API int ldpc_b200_sim_point(ldpc_b200_ctx *ctx, decoder_param dp, cons
  * (up to `capacity` records, unordered; *n_errors receives the number of frames in error, which may exceed capacity).
  * A record names the GLOBAL frame index: because the channel is counter-based, ldpc_b200_channel(frame0 = record.frame,
  * n = 1) regenerates that frame's decoder input exactly and ldpc_b200_decode_batch replays the decoding, which yields
- * the failed bit / check indices and the syndrome weight (libldpc_b200/api.py: Context.error_report).  All three channels. */
+ * the failed bit / check indices and the syndrome weight (libldpc_b200/api.py: Context.error_report).  All four channels. */
 typedef struct
 {
     uint64_t frame;      /* global frame index of the sweep point */
@@ -283,7 +291,7 @@ LDPC_B200_API int ldpc_b200_sim_point_async(ldpc_b200_ctx *ctx, decoder_param dp
                               uint32_t point, uint64_t frame0, uint64_t n_frames, uint64_t *d_counters, void *stream);
 
 /* Whole sweep with the reference's semantics (x list, reversed order for BSC/BEC, stop rule, results
- * file layout — src/sim/ldpcsim.cpp:97-263).  rank/world shard the frames of every round across
+ * file layout — src/sim/ldpcsim.cpp:97-263).  Channels "AWGN", "BSC", "BEC" and "RAYLEIGH" (ascending SNR like AWGN).  rank/world shard the frames of every round across
  * processes; `allreduce` (may be NULL when world == 1) is called once per round with a small host
  * array of uint64 counters to be summed over ranks (the caller wires it to NCCL/gloo).  quiet != 0 suppresses the console table. */
 typedef void (*ldpc_b200_allreduce_fn)(uint64_t *values, int n, void *user); /* in-place sum over ranks */

@@ -71,7 +71,7 @@ HANDLE_SYMBOLS = ("ldpc_b200_last_error", "ldpc_b200_version", "ldpc_b200_device
                   "ldpc_b200_decode_batch", "ldpc_b200_decode_batch_device", "ldpc_b200_decode_bec_batch", "ldpc_b200_channel",
                   "ldpc_b200_sim_point", "ldpc_b200_sim_point_async", "ldpc_b200_simulate", "ldpc_b200_simulate_ex", "ldpc_b200_get_stats",
                   "ldpc_b200_reset_stats", "ldpc_b200_smem_probe", "ldpc_b200_sim_point_log", "ldpc_b200_prepare", "ldpc_b200_decode_batch_ex", "ldpc_b200_decode_batch_device_ex", "ldpc_b200_get_bec_layout", "ldpc_b200_fp64_probe", "ldpc_b200_set_layers", "ldpc_b200_load_layers", "ldpc_b200_get_layers", "ldpc_b200_set_modulation",
-                  "ldpc_b200_error_report")
+                  "ldpc_b200_error_report", "ldpc_b200_set_fading")
 
 _lib = None
 
@@ -124,6 +124,7 @@ def load_library(path=None):
     L.ldpc_b200_get_layout.argtypes = [vp, iptr, iptr, iptr, iptr, iptr]
     L.ldpc_b200_get_bec_layout.argtypes = [vp, iptr, iptr]
     L.ldpc_b200_set_modulation.argtypes = [vp, ct.c_int, iptr, iptr]
+    L.ldpc_b200_set_fading.argtypes = [vp, ct.c_int]
     L.ldpc_b200_set_layers.argtypes = [vp, ct.c_int, iptr, iptr]
     L.ldpc_b200_load_layers.argtypes = [vp, ct.c_char_p]
     L.ldpc_b200_get_layers.argtypes = [vp, iptr]
@@ -223,6 +224,11 @@ class Context:
         lab = np.ascontiguousarray(labels, np.int32) if labels is not None else None
         bm = np.ascontiguousarray(bit_mapper, np.int32) if bit_mapper is not None else None
         self._check(self.lib.ldpc_b200_set_modulation(self._h, int(M), _p(lab, ct.c_int), _p(bm, ct.c_int)))
+
+    def set_fading(self, coherence=1):
+        """Coherence length of the "RAYLEIGH" channel: transmitted positions per fading coefficient (1: fast fading, 0: one
+        coefficient per frame)."""
+        self._check(self.lib.ldpc_b200_set_fading(self._h, int(coherence)))
 
     def set_layers(self, layers=None):
         """Layers of the layered schedule: a list of check-index lists, or None for the built-in first-fit layering."""

@@ -1,13 +1,13 @@
 // ldpcsim — command-line front end with the reference's interface (src/sim_cpu.cpp:7-22):
 //   ldpcsim [options] codefile output-file MIN MAX STEP
 //   -G/--gen-matrix FILE  -i/--num-iterations N (50)  -s/--seed N (0)  -t/--num-threads N (1, ignored)
-//   --channel AWGN|BSC|BEC (AWGN)  --decoding BP|BP_MS (BP)  --max-frames N (10e9)
+//   --channel AWGN|BSC|BEC (AWGN; B200 extra: RAYLEIGH)  --decoding BP|BP_MS (BP)  --max-frames N (10e9)
 //   --frame-error-count N (50)  --no-early-term  -h/--help  -v/--version
 // Negative MIN/MAX are positionals, as with the reference's argument parser.
 // B200 extras (do not exist in the reference): --precision f64|f32, --device N, --gpus N / --devices LIST (frames of every
 // round sharded over N GPUs of this process, one host thread per shard; the counters are summed on the host, results do not
 // depend on the number of shards), --error-log FILE (per sweep point, the first --frame-error-count frames in error, replayed on the
-// GPU: failed bits and checks; see the usage text).
+// GPU: failed bits and checks; see the usage text), --channel RAYLEIGH with --coherence L (flat Rayleigh fading, DESIGN.md §3.2).
 // The CLI is a client of the C ABI only (include/ldpc_b200.h): the library exports nothing else.
 #include <algorithm>
 #include <cstdio>
@@ -39,7 +39,8 @@ namespace
         "-i --num-iterations \tNumber of iterations for decoding. (Default: 50)\n"
         "-s --seed           \tRNG seed. (Default: 0)\n"
         "-t --num-threads    \tNumber of frames to be decoded in parallel. (Default: 1; ignored, the GPU batches frames)\n"
-        "--channel           \tSpecifies channel: \"AWGN\", \"BSC\", \"BEC\" (Default: AWGN)\n"
+        "--channel           \tSpecifies channel: \"AWGN\", \"BSC\", \"BEC\" (Default: AWGN); B200 only: \"RAYLEIGH\" (BPSK over flat Rayleigh\n"
+        "                    \tfading with perfect CSI at the receiver, x = average SNR in dB)\n"
         "--decoding          \tSpecifies decoding algorithm: \"BP\", \"BP_MS\" (Default: BP)\n"
         "--max-frames        \tLimit number of decoded frames.\n"
         "--frame-error-count \tMaximum frame errors for given simulation point.\n"
@@ -52,6 +53,8 @@ namespace
         "--modulation        \tB200 only: M-ASK with bit-metric decoding on the AWGN channel, M = 4, 8, ... (Gray labels, consecutive bit mapper; Default: 2 = BPSK)\n"
         "--layers            \tB200 only: layer file for --schedule layered (legacy format: nl: N / cn[i]: W / W check indices); default: built-in layering\n"
         "--devices           \tB200 only: explicit device list for the shards, e.g. 0,1,2,3 (an index may repeat: several shards on one GPU)\n"
+        "--coherence         \tB200 only: with --channel RAYLEIGH: transmitted bits per fading coefficient, >= 0 (Default: 1 = fast fading;\n"
+        "                    \t0 = one coefficient per frame)\n"
         "--error-log         \tB200 only: file of the frames in error: per point the first --frame-error-count of them in frame order, one line\n"
         "                    \teach: snr frame iterations bit_errors syndrome_weight failed_bits failed_checks (comma-separated lists, - = empty;\n"
         "                    \tsyndrome_weight 0 with bit_errors > 0 is an undetected error); written after every round\n";
@@ -230,6 +233,8 @@ int main(int argc, char **argv)
     std::string device_list, schedule = "flooding", layer_file, error_log;
     double ms_scale = 1.0;
     int modulation = 2;
+    int coherence = 1;
+    bool coherence_set = false;
     std::vector<std::string> pos;
     try
     {
@@ -261,6 +266,7 @@ int main(int argc, char **argv)
             else if (a == "--ms-scale") ms_scale = std::stod(value());
             else if (a == "--modulation") modulation = std::stoi(value());
             else if (a == "--error-log") error_log = value();
+            else if (a == "--coherence") { coherence = std::stoi(value()); coherence_set = true; }
             else if (a.size() > 1 && a[0] == '-' && !looks_numeric(a)) throw std::runtime_error("Unknown argument: " + a);
             else pos.push_back(a);
         }
@@ -270,6 +276,9 @@ int main(int argc, char **argv)
         if (snr[0] > snr[1]) throw std::runtime_error("snr min > snr max");
         if (precision != "f64" && precision != "f32") throw std::runtime_error("--precision must be f64 or f32");
         if (schedule != "flooding" && schedule != "layered") throw std::runtime_error("--schedule must be flooding or layered");
+        if (coherence_set && channel != "RAYLEIGH") throw std::runtime_error("--coherence applies to --channel RAYLEIGH only");
+        if (coherence < 0) throw std::runtime_error("--coherence must be >= 0");
+        if (channel == "RAYLEIGH" && modulation != 2) throw std::runtime_error("--channel RAYLEIGH is BPSK only: --modulation must be 2");
 
         std::vector<int> devices;
         if (!device_list.empty()) devices = parse_devices(device_list);
@@ -309,6 +318,11 @@ int main(int argc, char **argv)
         if (modulation != 2 && ldpc_b200_set_modulation(ctx, modulation, nullptr, nullptr) != 0)
         {
             std::cout << "Error: modulation: " << ldpc_b200_last_error() << std::endl;
+            return EXIT_FAILURE;
+        }
+        if (channel == "RAYLEIGH" && ldpc_b200_set_fading(ctx, coherence) != 0)
+        {
+            std::cout << "Error: fading: " << ldpc_b200_last_error() << std::endl;
             return EXIT_FAILURE;
         }
         if (!layer_file.empty() && ldpc_b200_load_layers(ctx, layer_file.c_str()) != 0)
@@ -360,8 +374,13 @@ int main(int argc, char **argv)
                 if (!c) { std::cout << "Error: ldpc_code(): " << ldpc_b200_last_error() << std::endl; return EXIT_FAILURE; }
                 ldpc_b200_set_tuning(c, &tn);
                 if (!layer_file.empty()) ldpc_b200_load_layers(c, layer_file.c_str());
+                m.ctxs.push_back(c); // closed with the others from here on
                 if (modulation != 2) ldpc_b200_set_modulation(c, modulation, nullptr, nullptr);
-                m.ctxs.push_back(c);
+                if (channel == "RAYLEIGH" && ldpc_b200_set_fading(c, coherence) != 0)
+                {
+                    std::cout << "Error: fading: GPU " << devices[g] << ": " << ldpc_b200_last_error() << std::endl;
+                    return EXIT_FAILURE;
+                }
             }
             if (devices.size() > 1)
             {

@@ -128,7 +128,7 @@ namespace b200
         // a persistent grid of `ctas` CTAs, but no more CTAs than work items (`need`) and at least one
         int clamp_grid(int ctas, uint64_t need) { return (uint64_t)ctas > need ? (int)std::max<uint64_t>(need, 1) : ctas; }
 
-        // Channel constants of a point: AWGN (and M-ASK) at x dB -> noise variance, deviation and LLR scale
+        // Channel constants of a point: AWGN (M-ASK, Rayleigh fading) at x dB -> noise variance, deviation and LLR scale
         // (src/sim/channel.cpp:39-40); BSC / BEC with probability x -> the BSC's LLR magnitude (src/sim/channel.cpp:139) and the
         // 32-bit threshold of a uniform word.  The other channel's fields stay 0.
         struct ChannelConsts
@@ -139,7 +139,7 @@ namespace b200
         ChannelConsts channel_consts(int kind, double x)
         {
             ChannelConsts c;
-            if (kind == SRC_AWGN || kind == SRC_ASK)
+            if (kind == SRC_AWGN || kind == SRC_ASK || kind == SRC_RAYLEIGH)
             {
                 c.sigma2 = std::pow(10.0, -x / 10.0);
                 c.sigma = std::sqrt(c.sigma2);
@@ -628,11 +628,16 @@ namespace b200
         return best;
     }
 
-    int Engine::channel_kind(const std::string &name)
+    int Engine::channel_kind(const std::string &name) const
     {
         if (name == "AWGN") return SRC_AWGN;
         if (name == "BSC") return SRC_BSC;
         if (name == "BEC") return SRC_BEC;
+        if (name == "RAYLEIGH")
+        {
+            if (ask_M > 2) throw std::runtime_error("the RAYLEIGH channel is BPSK only: set the modulation back to M = 2");
+            return SRC_RAYLEIGH;
+        }
         throw std::runtime_error("No channel selected."); // message of src/sim/ldpcsim.cpp:72
     }
 
@@ -677,6 +682,7 @@ namespace b200
         kp.early_term = dp.earlyTerm ? 1 : 0;
         kp.kind = (src.kind == SRC_AWGN && ask_M > 2) ? SRC_ASK : src.kind;
         if (kp.kind == SRC_ASK) ask_fill(&kp.ask);
+        kp.coherence = fading_L;
         kp.llr_in = src.d_llr; kp.llr_in_f32 = src.d_llr_f32; kp.llr_in_i8 = src.d_llr_i8; kp.i8_scale = src.i8_scale;
         const ChannelConsts cc = channel_consts(src.kind, src.x);
         kp.sigma2 = cc.sigma2; kp.sigma = cc.sigma; kp.llr_scale = cc.llr_scale; kp.delta = cc.delta; kp.thr = cc.thr;
@@ -992,6 +998,7 @@ namespace b200
         lp.nc = H.nc; lp.nct = H.nct(); lp.n_punct = (int)H.puncture.size(); lp.n_short = (int)H.shorten.size();
         lp.tx_var = d_bit_pos_.get(); lp.punct = d_punct_.get(); lp.shorten = d_short_.get();
         lp.max_iter = (int)dp.iterations; lp.early_term = dp.earlyTerm ? 1 : 0; lp.kind = src.kind;
+        lp.coherence = fading_L;
         lp.llr_in = src.d_llr;
         const ChannelConsts cc = channel_consts(src.kind, src.x);
         lp.sigma = cc.sigma; lp.llr_scale = cc.llr_scale; lp.delta = cc.delta; lp.thr = cc.thr;
@@ -1388,7 +1395,7 @@ namespace b200
                                    const int32_t *__restrict__ shorten, int n_short, double sigma, double llr_scale, double delta, uint32_t thr,
                                    uint64_t seed, uint32_t point, uint64_t frame0, int64_t n_frames, uint8_t *cw, double *llr, uint8_t *llr_u8,
                                    const int32_t *__restrict__ g_col_ptr, const int32_t *__restrict__ g_row, int g_rows, int g_cols, AskParams ask,
-                                   double sigma2, const uint64_t *__restrict__ frames)
+                                   double sigma2, const uint64_t *__restrict__ frames, int coherence)
     {
         auto frame_of = [&](int64_t fr) -> uint64_t { return GATHER ? frames[fr] : frame0 + fr; };
         if (kind == SRC_ASK)
@@ -1456,6 +1463,22 @@ namespace b200
                     if (cw) cw[base + bit_pos[t]] = (uint8_t)b;
                 }
             }
+            else if (kind == SRC_RAYLEIGH)
+            { // the same arithmetic as the fused path (tile4.cuh frame_pass)
+                float z[4];
+                normal_pair(r.x, r.y, z[0], z[1]);
+                normal_pair(r.z, r.w, z[2], z[3]);
+                for (int q = 0; q < 4; ++q)
+                {
+                    const int t = j + q * nblk;
+                    if (t >= nct) break;
+                    const uint32_t b = cw_bit(fr, bit_pos[t]);
+                    const double h = rayleigh_coeff(seed, point, frame_of(fr), coherence ? (uint32_t)(t / coherence) : 0u);
+                    const double y = __dadd_rn(__dmul_rn((double)z[q], sigma), b ? -h : h);
+                    llr[base + bit_pos[t]] = __dmul_rn(__dmul_rn(y, h), llr_scale);
+                    if (cw) cw[base + bit_pos[t]] = (uint8_t)b;
+                }
+            }
             else
             {
                 const uint32_t w[4] = {r.x, r.y, r.z, r.w};
@@ -1488,7 +1511,7 @@ namespace b200
                 for (int i = 0; i < n_short; ++i)
                 {
                     if (kind == SRC_BEC) llr_u8[base + shorten[i]] = (uint8_t)cw_bit(fr, shorten[i]); // the true bit (channel.cpp:219-222)
-                    else llr[base + shorten[i]] = (kind == SRC_AWGN) ? 99999.9 : delta;
+                    else llr[base + shorten[i]] = (kind == SRC_BSC) ? delta : 99999.9;
                 }
                 if (cw)
                 { // non-transmitted positions carry their codeword bit too
@@ -1500,7 +1523,7 @@ namespace b200
     }
 
     // Enqueues the channel kernel on s: rows of global frames frame0 + fr, or frames[fr] when `frames` (device) is given.
-    // kind = SRC_AWGN is M-ASK under the current modulation.
+    // kind = SRC_AWGN is M-ASK under the current modulation; SRC_RAYLEIGH uses the context's coherence length.
     void Engine::launch_channel(int kind, double x, uint64_t seed, uint32_t point, uint64_t frame0, const uint64_t *frames, int64_t n,
                                 uint8_t *d_cw, double *d_llr, uint8_t *d_u8, cudaStream_t s)
     {
@@ -1511,7 +1534,7 @@ namespace b200
         auto fn = frames ? channel_kernel<true> : channel_kernel<false>;
         fn<<<sm_count_ * 4, 256, 0, s>>>(kind, H.nc, H.nct(), d_bit_pos_.get(), d_punct_.get(), (int)H.puncture.size(), d_short_.get(),
                                          (int)H.shorten.size(), cc.sigma, cc.llr_scale, cc.delta, cc.thr, seed, point, frame0, n, d_cw, d_llr, d_u8,
-                                         d_g_col_ptr_.get(), d_g_row_.get(), g_rows, g_cols, ask, cc.sigma2, frames);
+                                         d_g_col_ptr_.get(), d_g_row_.get(), g_rows, g_cols, ask, cc.sigma2, frames, fading_L);
         CUDA_OK(cudaGetLastError());
     }
 

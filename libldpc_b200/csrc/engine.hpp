@@ -7,6 +7,7 @@
 #include <map>
 #include <memory>
 #include <set>
+#include <stdexcept>
 #include <string>
 #include <tuple>
 #include <vector>
@@ -121,6 +122,14 @@ namespace b200
         std::vector<int32_t> ask_labels, ask_rev, ask_bm;
         std::vector<double> ask_X;
 
+        // Rayleigh fading: transmitted positions per fading coefficient (0 = one coefficient per frame, quasi-static)
+        void set_fading(int coherence)
+        {
+            if (coherence < 0) throw std::runtime_error("fading: the coherence length must be >= 0");
+            fading_L = coherence;
+        }
+        int fading_L = 1;
+
         // layered schedule: the layering in use (empty = built-in first-fit layering, made on first use)
         void set_layers(std::vector<std::vector<int>> layers);
         const std::vector<std::vector<int>> &layers();
@@ -170,7 +179,7 @@ namespace b200
         void ensure_state(size_t bytes, CUstream_st *s);
         void release_state(CUstream_st *s);
         bool try_seg_layout(int lanes, int threads, int isz);
-        static int channel_kind(const std::string &name);
+        int channel_kind(const std::string &name) const; // SRC_* of a channel name; RAYLEIGH needs BPSK
         void launch_channel(int kind, double x, uint64_t seed, uint32_t point, uint64_t frame0, const uint64_t *frames, int64_t n,
                             uint8_t *d_cw, double *d_llr, uint8_t *d_u8, CUstream_st *s);
         const void *tile_fn(const Config &c, bool et); // the tile kernel of c (early termination: et), its attributes set

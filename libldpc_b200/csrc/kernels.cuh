@@ -83,7 +83,20 @@ namespace b200
         z1 = __fmul_rn(r, sn);
     }
 
-    enum { SRC_LLR = 0, SRC_AWGN = 1, SRC_BSC = 2, SRC_BEC = 3, SRC_ASK = 4 }; // SRC_ASK: AWGN with M-ASK + bit-metric decoding
+    // Rayleigh fading coefficient c of a frame (DESIGN.md §3.2): the first normal pair (a, b) of Philox block c of stream 3,
+    // h = sqrt((a^2 + b^2) / 2) in fp64, so E[h^2] = 1.  The squares of binary32 values are exact in fp64, the sum is rounded
+    // once, the halving is exact and the square root is correctly rounded: the oracle's sqrt gives the same bits.
+    __device__ __forceinline__ double rayleigh_coeff(uint64_t seed, uint32_t point, uint64_t frame, uint32_t c)
+    {
+        const u32x4 r = channel_block(seed, point, 3, frame, c);
+        float a, b;
+        normal_pair(r.x, r.y, a, b);
+        const double s = __dadd_rn(__dmul_rn((double)a, (double)a), __dmul_rn((double)b, (double)b));
+        return __dsqrt_rn(__dmul_rn(0.5, s));
+    }
+
+    // SRC_ASK: AWGN with M-ASK + bit-metric decoding; SRC_RAYLEIGH: BPSK over flat Rayleigh fading, perfect CSI
+    enum { SRC_LLR = 0, SRC_AWGN = 1, SRC_BSC = 2, SRC_BEC = 3, SRC_ASK = 4, SRC_RAYLEIGH = 5 };
 
     // M-ASK with bit-metric decoding (legacy tree gpu/device/kernel.cpp:141-219, gpu/sim/ldpcsim.cpp:240-323; specification:
     // oracle/ldpc_oracle.c orc_channel_frame_ask).  Tables in global memory.

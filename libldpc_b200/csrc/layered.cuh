@@ -26,6 +26,7 @@ namespace b200
         int n_layers, max_segs, n_slots, nc, nct, n_punct, n_short;
         const int32_t *tx_var, *punct, *shorten; // variable ids
         int max_iter, early_term, kind;
+        int coherence; // SRC_RAYLEIGH: transmitted positions per fading coefficient (0: one per frame)
         const double *llr_in;
         double sigma, llr_scale, delta;
         double ms_scale; // normalisation factor of the min-sum check output (1 = the reference's plain min-sum)
@@ -291,6 +292,20 @@ namespace b200
                         for (int k = 0; k < 4; ++k)
                             if (q + k * nblk < p.nct) put(p.tx_var[q + k * nblk], (T)__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), 1.0), p.llr_scale));
                     }
+                    else if (p.kind == SRC_RAYLEIGH)
+                    {
+                        float z[4];
+                        normal_pair(r.x, r.y, z[0], z[1]);
+                        normal_pair(r.z, r.w, z[2], z[3]);
+#pragma unroll
+                        for (int k = 0; k < 4; ++k)
+                        {
+                            const int t = q + k * nblk;
+                            if (t >= p.nct) continue;
+                            const double h = rayleigh_coeff(p.seed, p.point, frame, p.coherence ? (uint32_t)(t / p.coherence) : 0u);
+                            put(p.tx_var[t], (T)__dmul_rn(__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), h), h), p.llr_scale));
+                        }
+                    }
                     else
                     {
                         const uint32_t w[4] = {r.x, r.y, r.z, r.w};
@@ -300,7 +315,7 @@ namespace b200
                     }
                 }
                 for (int i = tid; i < p.n_punct; i += nthreads) put(p.punct[i], T(0));
-                for (int i = tid; i < p.n_short; i += nthreads) put(p.shorten[i], (T)(p.kind == SRC_AWGN ? 99999.9 : p.delta));
+                for (int i = tid; i < p.n_short; i += nthreads) put(p.shorten[i], (T)(p.kind == SRC_BSC ? p.delta : 99999.9));
             }
             __syncthreads();
 

@@ -228,6 +228,14 @@ extern "C"
         });
     }
 
+    int ldpc_b200_set_fading(ldpc_b200_ctx *ctx, int coherence)
+    {
+        return guarded([&] {
+            if (!ctx) throw std::runtime_error("null argument");
+            ctx->eng->set_fading(coherence);
+        });
+    }
+
     int ldpc_b200_set_layers(ldpc_b200_ctx *ctx, int n_layers, const int *layer_ptr, const int *layer_check)
     {
         return guarded([&] {

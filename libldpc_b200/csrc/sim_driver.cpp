@@ -23,7 +23,7 @@ namespace b200
                   void *user, bool quiet, bool write_file, ldpc_b200_round_fn round_fn)
     {
         const std::string ch = cp.type ? cp.type : "";
-        if (ch != "AWGN" && ch != "BSC" && ch != "BEC") throw std::runtime_error("No channel selected.");
+        if (ch != "AWGN" && ch != "BSC" && ch != "BEC" && ch != "RAYLEIGH") throw std::runtime_error("No channel selected.");
         if (world < 1 || rank < 0 || rank >= world) throw std::runtime_error("bad rank/world");
         if (world > 1 && !allreduce) throw std::runtime_error("world > 1 needs an allreduce callback");
 

@@ -224,6 +224,7 @@ namespace b200
         int max_iter, early_term;
         // frame source
         int kind;
+        int coherence; // SRC_RAYLEIGH: transmitted positions per fading coefficient (0: one per frame)
         const double *llr_in; // SRC_LLR: [n_frames][nc]; or one of the narrow encodings below (exactly one of the three is set)
         const float *llr_in_f32;  // widened exactly to the decoder's type
         const int8_t *llr_in_i8;  // quantised LLRs: value = i8 * i8_scale, evaluated in double (exact for a power-of-two scale)
@@ -924,6 +925,21 @@ namespace b200
                                 put(pos[k], (T)__dmul_rn(y, p.llr_scale));
                             }
                     }
+                    else if (p.kind == SRC_RAYLEIGH)
+                    { // the AWGN noise with the faded amplitude h: y = sigma*z + h*x, LLR = y*h*(2/sigma^2) (DESIGN.md §3.2)
+                        float z[4];
+                        normal_pair(r.x, r.y, z[0], z[1]);
+                        normal_pair(r.z, r.w, z[2], z[3]);
+#pragma unroll
+                        for (int k = 0; k < 4; ++k)
+                            if (ok[k])
+                            {
+                                const int t = q + k * nblk;
+                                const double h = rayleigh_coeff(p.seed, p.point, frame, p.coherence ? (uint32_t)(t / p.coherence) : 0u);
+                                const double y = __dadd_rn(__dmul_rn((double)z[k], p.sigma), (has_g && cw_bit(g, t)) ? -h : h);
+                                put(pos[k], (T)__dmul_rn(__dmul_rn(y, h), p.llr_scale));
+                            }
+                    }
                     else
                     { // BSC: y = x ^ Bernoulli(eps), LLR = delta*(1-2y) (src/sim/channel.cpp:123-162)
                         const uint32_t w[4] = {r.x, r.y, r.z, r.w};
@@ -939,7 +955,7 @@ namespace b200
 #endif
             if (gen)
             {
-                const T sv = (T)(p.kind == SRC_AWGN ? 99999.9 : p.delta);
+                const T sv = (T)(p.kind == SRC_BSC ? p.delta : 99999.9);
                 if constexpr (SMEM)
                 {
                     for (int i = tid; i < p.n_punct; i += nthreads) put((int)lds_u16<0>(a_pu + 2 * i), T(0));
