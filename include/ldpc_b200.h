@@ -102,6 +102,7 @@ LDPC_B200_API void syndrome(uint8_t *word, uint8_t *syndrome);
 typedef struct ldpc_b200_ctx ldpc_b200_ctx;
 
 enum { LDPC_B200_F64 = 0, LDPC_B200_F32 = 1 };          /* arithmetic / message type of the decoder */
+enum { LDPC_B200_FIXED = 2 }; /* ldpc_b200_stats.precision of the fixed-point layered decoder (ldpc_b200_set_quant); not a tuning value */
 enum { LDPC_B200_AUTO = 0, LDPC_B200_SMEM = 1, LDPC_B200_GLOBAL = 2 }; /* message residency */
 
 typedef struct
@@ -185,6 +186,27 @@ LDPC_B200_API int ldpc_b200_set_modulation(ldpc_b200_ctx *ctx, int M, const int 
  * normal pair of Philox block c of stream 3, E[h^2] = 1; y = sigma z + h (1 - 2 cw) with the AWGN channel's noise z at average
  * SNR x dB, LLR = y h 2 / sigma^2 (DESIGN.md 3.2).  Per context; negative values fail.  RAYLEIGH with M-ASK (M > 2) fails. */
 LDPC_B200_API int ldpc_b200_set_fading(ldpc_b200_ctx *ctx, int coherence);
+
+/* Fixed-point layered min-sum (not in the reference; DESIGN.md 3.7), the decoder of a hardware implementation: the fp64 channel
+ * LLR L (the channel's own, or the caller's for the batch decode) enters as clamp(round(L / step), -M(ch_bits), M(ch_bits)) with
+ * M(q) = 2^(q-1) - 1, round half away from zero; the check-to-variable messages have msg_bits and the posteriors post_bits, with
+ * saturating int32 arithmetic; a check sends sign * max(floor(m * scale8 / 8) - offset, 0), m = the smallest magnitude of the other
+ * edges clipped to M(msg_bits).  Valid: 2 <= msg_bits <= post_bits <= 16, 2 <= ch_bits <= post_bits, 0 <= offset < M(msg_bits),
+ * 1 <= scale8 <= 8, step > 0.  Decisions are P <= 0; llr_out receives P * step.
+ * Per context.  q = NULL or ch_bits = 0 turns it off; invalid parameters fail and keep the previous setting.  While it is on, the
+ * layered schedule (tuning.schedule = LDPC_B200_LAYERED, tuning.precision ignored) runs the int16 kernel: 16 or 32 frames per CTA
+ * (tuning.frames_per_cta 0 = 32), ldpc_b200_get_stats reports precision = LDPC_B200_FIXED, and no kernel-shape trial runs.  Every
+ * decoding entry point fails while it is on with the flooding schedule, decoder type BP, the BEC, M-ASK (M > 2), the narrow
+ * encodings of the batch decode or another frames_per_cta. */
+typedef struct
+{
+    int ch_bits, msg_bits, post_bits; /* bits of the channel LLR, of the check-to-variable messages and of the posterior */
+    int offset;                       /* beta, in LSBs */
+    int scale8;                       /* normalisation factor scale8 / 8 */
+    double step;                      /* LLR value of one LSB */
+} ldpc_b200_quant;
+LDPC_B200_API int ldpc_b200_set_quant(ldpc_b200_ctx *ctx, const ldpc_b200_quant *q);
+LDPC_B200_API int ldpc_b200_get_quant(const ldpc_b200_ctx *ctx, ldpc_b200_quant *q); /* ch_bits = 0: off */
 
 /* host-side views of the loaded code (file order; sizes from ldpc_b200_info) */
 LDPC_B200_API int ldpc_b200_get_edges(const ldpc_b200_ctx *ctx, int *rows /*[nnz]*/, int *cols /*[nnz]*/);

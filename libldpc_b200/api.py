@@ -42,6 +42,11 @@ class tuning(ct.Structure):
     _fields_ = [(k, ct.c_int) for k in ("precision", "residency", "frames_per_cta", "threads_per_cta", "ctas", "bec_deg1_compat", "tmem", "idx16", "zero_codeword", "schedule", "layered_ms_scale64")]
 
 
+class quant(ct.Structure):  # ldpc_b200_quant
+    _fields_ = [("ch_bits", ct.c_int), ("msg_bits", ct.c_int), ("post_bits", ct.c_int), ("offset", ct.c_int), ("scale8", ct.c_int),
+                ("step", ct.c_double)]
+
+
 class error_record(ct.Structure):  # ldpc_b200_error_record
     _fields_ = [("frame", ct.c_uint64), ("bit_errors", ct.c_uint32), ("iterations", ct.c_int32)]
 
@@ -60,6 +65,7 @@ class stats(ct.Structure):
 ALLREDUCE_FN = ct.CFUNCTYPE(None, ct.POINTER(ct.c_uint64), ct.c_int, ct.c_void_p)
 ROUND_FN = ct.CFUNCTYPE(ct.c_int, ct.c_uint32, ct.c_double, ct.c_uint64, ct.c_uint64, ct.POINTER(ct.c_uint64), ct.c_void_p)
 F64, F32 = 0, 1
+FIXED = 2  # stats()["precision"] of the fixed-point layered decoder (Context.set_quant)
 AUTO, SMEM, GLOBAL = 0, 1, 2
 LLR_F64, LLR_F32, LLR_I8 = 0, 1, 2
 FLOODING, LAYERED = 0, 1
@@ -71,7 +77,7 @@ HANDLE_SYMBOLS = ("ldpc_b200_last_error", "ldpc_b200_version", "ldpc_b200_device
                   "ldpc_b200_decode_batch", "ldpc_b200_decode_batch_device", "ldpc_b200_decode_bec_batch", "ldpc_b200_channel",
                   "ldpc_b200_sim_point", "ldpc_b200_sim_point_async", "ldpc_b200_simulate", "ldpc_b200_simulate_ex", "ldpc_b200_get_stats",
                   "ldpc_b200_reset_stats", "ldpc_b200_smem_probe", "ldpc_b200_sim_point_log", "ldpc_b200_prepare", "ldpc_b200_decode_batch_ex", "ldpc_b200_decode_batch_device_ex", "ldpc_b200_get_bec_layout", "ldpc_b200_fp64_probe", "ldpc_b200_set_layers", "ldpc_b200_load_layers", "ldpc_b200_get_layers", "ldpc_b200_set_modulation",
-                  "ldpc_b200_error_report", "ldpc_b200_set_fading")
+                  "ldpc_b200_error_report", "ldpc_b200_set_fading", "ldpc_b200_set_quant", "ldpc_b200_get_quant")
 
 _lib = None
 
@@ -125,6 +131,8 @@ def load_library(path=None):
     L.ldpc_b200_get_bec_layout.argtypes = [vp, iptr, iptr]
     L.ldpc_b200_set_modulation.argtypes = [vp, ct.c_int, iptr, iptr]
     L.ldpc_b200_set_fading.argtypes = [vp, ct.c_int]
+    L.ldpc_b200_set_quant.argtypes = [vp, ct.POINTER(quant)]
+    L.ldpc_b200_get_quant.argtypes = [vp, ct.POINTER(quant)]
     L.ldpc_b200_set_layers.argtypes = [vp, ct.c_int, iptr, iptr]
     L.ldpc_b200_load_layers.argtypes = [vp, ct.c_char_p]
     L.ldpc_b200_get_layers.argtypes = [vp, iptr]
@@ -229,6 +237,24 @@ class Context:
         """Coherence length of the "RAYLEIGH" channel: transmitted positions per fading coefficient (1: fast fading, 0: one
         coefficient per frame)."""
         self._check(self.lib.ldpc_b200_set_fading(self._h, int(coherence)))
+
+    def set_quant(self, ch_bits, msg_bits=None, post_bits=None, step=None, offset=0, scale8=8):
+        """Fixed-point layered min-sum (DESIGN.md §3.7): channel LLRs quantised to ch_bits with LSB `step`, msg_bits check-to-variable
+        messages, post_bits posteriors, offset beta in LSBs and normalisation factor scale8 / 8.  set_quant(None) turns it off.
+        Needs the layered schedule and BP_MS."""
+        if ch_bits is None or ch_bits == 0:
+            self._check(self.lib.ldpc_b200_set_quant(self._h, None))
+            return
+        if msg_bits is None or post_bits is None or step is None:
+            raise ValueError("set_quant needs ch_bits, msg_bits, post_bits and step")
+        q = quant(int(ch_bits), int(msg_bits), int(post_bits), int(offset), int(scale8), float(step))
+        self._check(self.lib.ldpc_b200_set_quant(self._h, ct.byref(q)))
+
+    def quant(self):
+        """The fixed-point setting as a dict, or None when it is off."""
+        q = quant()
+        self._check(self.lib.ldpc_b200_get_quant(self._h, ct.byref(q)))
+        return {k: getattr(q, k) for k, _ in quant._fields_} if q.ch_bits else None
 
     def set_layers(self, layers=None):
         """Layers of the layered schedule: a list of check-index lists, or None for the built-in first-fit layering."""

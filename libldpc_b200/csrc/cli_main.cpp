@@ -7,9 +7,11 @@
 // B200 extras (do not exist in the reference): --precision f64|f32, --device N, --gpus N / --devices LIST (frames of every
 // round sharded over N GPUs of this process, one host thread per shard; the counters are summed on the host, results do not
 // depend on the number of shards), --error-log FILE (per sweep point, the first --frame-error-count frames in error, replayed on the
-// GPU: failed bits and checks; see the usage text), --channel RAYLEIGH with --coherence L (flat Rayleigh fading, DESIGN.md §3.2).
+// GPU: failed bits and checks; see the usage text), --channel RAYLEIGH with --coherence L (flat Rayleigh fading, DESIGN.md §3.2),
+// --quantize CH,MSG,POST --llr-step D [--ms-offset B] (fixed-point layered min-sum, DESIGN.md §3.7).
 // The CLI is a client of the C ABI only (include/ldpc_b200.h): the library exports nothing else.
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <array>
@@ -57,7 +59,12 @@ namespace
         "                    \t0 = one coefficient per frame)\n"
         "--error-log         \tB200 only: file of the frames in error: per point the first --frame-error-count of them in frame order, one line\n"
         "                    \teach: snr frame iterations bit_errors syndrome_weight failed_bits failed_checks (comma-separated lists, - = empty;\n"
-        "                    \tsyndrome_weight 0 with bit_errors > 0 is an undetected error); written after every round\n";
+        "                    \tsyndrome_weight 0 with bit_errors > 0 is an undetected error); written after every round\n"
+        "--quantize          \tB200 only: fixed-point layered min-sum with CH,MSG,POST bits of the channel LLR, the check-to-variable messages\n"
+        "                    \tand the posterior (2 <= MSG <= POST <= 16, 2 <= CH <= POST); needs --schedule layered, --decoding BP_MS and\n"
+        "                    \t--llr-step; not on the BEC or with --modulation > 2.  --ms-scale is then a multiple of 1/8\n"
+        "--llr-step          \tB200 only: with --quantize: LLR value of one LSB (> 0); channel LLRs enter as clamp(round(L / step))\n"
+        "--ms-offset         \tB200 only: with --quantize: min-sum offset in LSBs, 0 <= B < 2^(MSG-1) - 1 (Default: 0)\n";
 
     bool looks_numeric(const std::string &s)
     {
@@ -235,6 +242,10 @@ int main(int argc, char **argv)
     int modulation = 2;
     int coherence = 1;
     bool coherence_set = false;
+    std::string quantize;
+    double llr_step = 0;
+    int ms_offset = 0;
+    bool llr_step_set = false, ms_offset_set = false, ms_scale_set = false;
     std::vector<std::string> pos;
     try
     {
@@ -263,10 +274,13 @@ int main(int argc, char **argv)
             else if (a == "--devices") device_list = value();
             else if (a == "--schedule") schedule = value();
             else if (a == "--layers") layer_file = value();
-            else if (a == "--ms-scale") ms_scale = std::stod(value());
+            else if (a == "--ms-scale") { ms_scale = std::stod(value()); ms_scale_set = true; }
             else if (a == "--modulation") modulation = std::stoi(value());
             else if (a == "--error-log") error_log = value();
             else if (a == "--coherence") { coherence = std::stoi(value()); coherence_set = true; }
+            else if (a == "--quantize") quantize = value();
+            else if (a == "--llr-step") { llr_step = std::stod(value()); llr_step_set = true; }
+            else if (a == "--ms-offset") { ms_offset = std::stoi(value()); ms_offset_set = true; }
             else if (a.size() > 1 && a[0] == '-' && !looks_numeric(a)) throw std::runtime_error("Unknown argument: " + a);
             else pos.push_back(a);
         }
@@ -279,6 +293,32 @@ int main(int argc, char **argv)
         if (coherence_set && channel != "RAYLEIGH") throw std::runtime_error("--coherence applies to --channel RAYLEIGH only");
         if (coherence < 0) throw std::runtime_error("--coherence must be >= 0");
         if (channel == "RAYLEIGH" && modulation != 2) throw std::runtime_error("--channel RAYLEIGH is BPSK only: --modulation must be 2");
+        ldpc_b200_quant qt{};
+        if (quantize.empty())
+        {
+            if (llr_step_set) throw std::runtime_error("--llr-step applies to --quantize only");
+            if (ms_offset_set) throw std::runtime_error("--ms-offset applies to --quantize only");
+        }
+        else
+        {
+            if (schedule != "layered") throw std::runtime_error("--quantize needs --schedule layered");
+            if (decoding != "BP_MS") throw std::runtime_error("--quantize needs --decoding BP_MS");
+            if (channel == "BEC") throw std::runtime_error("--quantize does not apply to --channel BEC");
+            if (modulation != 2) throw std::runtime_error("--quantize needs --modulation 2");
+            if (!llr_step_set) throw std::runtime_error("--quantize needs --llr-step");
+            if (!(llr_step > 0)) throw std::runtime_error("--llr-step must be > 0");
+            if (std::sscanf(quantize.c_str(), "%d,%d,%d", &qt.ch_bits, &qt.msg_bits, &qt.post_bits) != 3 ||
+                std::count(quantize.begin(), quantize.end(), ',') != 2)
+                throw std::runtime_error("--quantize expects CH,MSG,POST (three bit widths)");
+            if (!(qt.msg_bits >= 2 && qt.msg_bits <= qt.post_bits && qt.post_bits <= 16 && qt.ch_bits >= 2 && qt.ch_bits <= qt.post_bits))
+                throw std::runtime_error("--quantize: bit widths must satisfy 2 <= MSG <= POST <= 16 and 2 <= CH <= POST");
+            if (ms_offset < 0 || ms_offset >= (1 << (qt.msg_bits - 1)) - 1) throw std::runtime_error("--ms-offset must be >= 0 and < 2^(MSG-1) - 1");
+            const double a8 = ms_scale * 8.0;
+            if (ms_scale_set && !(a8 >= 1 && a8 <= 8 && a8 == std::floor(a8))) throw std::runtime_error("--ms-scale must be a multiple of 1/8 in [1/8, 1] with --quantize");
+            qt.offset = ms_offset;
+            qt.scale8 = ms_scale_set ? (int)a8 : 8;
+            qt.step = llr_step;
+        }
 
         std::vector<int> devices;
         if (!device_list.empty()) devices = parse_devices(device_list);
@@ -330,6 +370,11 @@ int main(int argc, char **argv)
             std::cout << "Error: layers: " << ldpc_b200_last_error() << std::endl;
             return EXIT_FAILURE;
         }
+        if (qt.ch_bits && ldpc_b200_set_quant(ctx, &qt) != 0)
+        {
+            std::cout << "Error: quantize: " << ldpc_b200_last_error() << std::endl;
+            return EXIT_FAILURE;
+        }
         ldpc_b200_code_info H;
         ldpc_b200_info(ctx, &H);
         std::vector<int> puncture(std::max(H.n_punct, 1)), shorten(std::max(H.n_short, 1));
@@ -359,6 +404,9 @@ int main(int argc, char **argv)
                   << ", Step: " << cp.xRange[2] << "\n";
         if (tn.schedule == LDPC_B200_LAYERED)
             std::cout << "== Schedule\n layered (" << ldpc_b200_get_layers(ctx, nullptr) << " layers" << (layer_file.empty() ? ", built-in layering" : (", " + layer_file)) << ")\n";
+        if (qt.ch_bits)
+            std::cout << "== Fixed point\n bits (channel, message, posterior): " << qt.ch_bits << ", " << qt.msg_bits << ", " << qt.post_bits << "\n LLR step: " << qt.step
+                      << "\n Offset: " << qt.offset << "\n Scale: " << qt.scale8 << "/8\n";
         std::cout << "== Simulation Parameters\n Threads: " << sp.threads << "\n FEC: " << sp.fec << "\n Max Frames: " << sp.maxFrames
                   << "\n Output File: " << sp.resultFile << "\n" << std::endl;
         std::cout << bar << std::endl;
@@ -379,6 +427,11 @@ int main(int argc, char **argv)
                 if (channel == "RAYLEIGH" && ldpc_b200_set_fading(c, coherence) != 0)
                 {
                     std::cout << "Error: fading: GPU " << devices[g] << ": " << ldpc_b200_last_error() << std::endl;
+                    return EXIT_FAILURE;
+                }
+                if (qt.ch_bits && ldpc_b200_set_quant(c, &qt) != 0)
+                {
+                    std::cout << "Error: quantize: GPU " << devices[g] << ": " << ldpc_b200_last_error() << std::endl;
                     return EXIT_FAILURE;
                 }
             }

@@ -647,6 +647,15 @@ namespace b200
         ensure_cuda();
         cudaStream_t s = stream ? (cudaStream_t)stream : stream_.get();
         if (dp.iterations == 0) throw std::runtime_error("iterations must be >= 1");
+        if (quantised())
+        { // the fixed-point decoder is layered min-sum on BPSK frames with fp64 LLRs: anything else is an error, not a fallback
+            if (tuning.schedule != LDPC_B200_LAYERED) throw std::runtime_error("quantised decoding runs on the layered schedule only (tuning.schedule = LDPC_B200_LAYERED)");
+            if (src.kind == SRC_BEC || src.d_bec_in) throw std::runtime_error("quantised decoding does not apply to the BEC");
+            if (alg_of(dp) != ALG_MS) throw std::runtime_error("quantised decoding is min-sum only (decoder type BP_MS)");
+            if (src.kind == SRC_AWGN && ask_M > 2) throw std::runtime_error("quantised decoding is BPSK only: set the modulation back to M = 2");
+            if (src.d_llr_f32 || src.d_llr_i8 || sink.d_hard_bits)
+                throw std::runtime_error("quantised decoding takes fp64 LLRs and byte decisions: the narrow encodings are not supported");
+        }
 
         if (src.kind == SRC_BEC || src.d_bec_in)
         {
@@ -779,6 +788,7 @@ namespace b200
 
     void Engine::maybe_autotune(int alg, const decoder_param &dp, uint64_t n_frames, cudaStream_t s)
     {
+        if (quantised()) return; // the fixed-point kernel has one shape: no trial, and nothing stored under a flooding key
         tune_cache_load();
         const auto key = std::make_pair(tuning.precision, alg);
         if (in_autotune_ || n_frames < 20000 || tuning.frames_per_cta > 0 || tuning.threads_per_cta > 0 || tuned_.count(key) || pair_tuned_.count(key)) return;
@@ -970,14 +980,20 @@ namespace b200
         if (src.kind == SRC_AWGN && ask_M > 2) throw std::runtime_error("layered schedule: higher-order modulation is served by the flooding path only");
         if (has_gen && !tuning.zero_codeword && src.kind != SRC_LLR)
             throw std::runtime_error("layered schedule: sweeps transmit the all-zero codeword (set tuning.zero_codeword = 1 with a generator matrix loaded)");
-        const int vec = tuning.precision == LDPC_B200_F32 ? 4 : 2;
-        int lanes = 4;
-        if (tuning.frames_per_cta > 0)
+        const bool q = quantised();
+        const int vec = q ? 8 : tuning.precision == LDPC_B200_F32 ? 4 : 2;
+        int lanes = 4, threads = 0, per_sm = 0;
+        const void *fn = nullptr;
+        if (q) quant_shape(&lanes, &threads, &fn, &per_sm);
+        else
         {
-            if (tuning.frames_per_cta != 2 * vec && tuning.frames_per_cta != 4 * vec) throw std::runtime_error("layered schedule: frames_per_cta / vector width must be 2 or 4");
-            lanes = tuning.frames_per_cta / vec;
+            if (tuning.frames_per_cta > 0)
+            {
+                if (tuning.frames_per_cta != 2 * vec && tuning.frames_per_cta != 4 * vec) throw std::runtime_error("layered schedule: frames_per_cta / vector width must be 2 or 4");
+                lanes = tuning.frames_per_cta / vec;
+            }
+            threads = tuning.threads_per_cta > 0 ? std::min(tuning.threads_per_cta, 512) : 256;
         }
-        const int threads = tuning.threads_per_cta > 0 ? std::min(tuning.threads_per_cta, 512) : 256;
         auto key = std::make_pair(lanes, threads);
         auto it = dev_lay_.find(key);
         if (it == dev_lay_.end())
@@ -1007,10 +1023,18 @@ namespace b200
         lp.llr_out = sink.d_llr_out; lp.hard_out = sink.d_hard; lp.iters_out = sink.d_iters;
         lp.counters = sink.d_counters ? sink.d_counters : d_counters_.get();
         lp.err_log = sink.d_err_log; lp.err_count = sink.d_err_count; lp.err_cap = sink.err_cap;
+        if (q)
+        {
+            lp.q_step = quant.step;
+            lp.q_ch_max = (1 << (quant.ch_bits - 1)) - 1; lp.q_msg_max = (1 << (quant.msg_bits - 1)) - 1; lp.q_post_max = (1 << (quant.post_bits - 1)) - 1;
+            lp.q_offset = quant.offset; lp.q_scale8 = quant.scale8;
+        }
         const int fpc = lanes * vec;
-        const void *fn = layered_kernel(tuning.precision == LDPC_B200_F32, alg_of(dp), lanes);
-        int per_sm = 0;
-        CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, 0));
+        if (!q)
+        {
+            fn = layered_kernel(tuning.precision == LDPC_B200_F32, alg_of(dp), lanes);
+            CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, 0));
+        }
         if (per_sm < 1) throw std::runtime_error("layered kernel does not fit on this device");
         const int ctas = clamp_grid(tuning.ctas > 0 ? tuning.ctas : sm_count_ * per_sm, (n_frames + fpc - 1) / fpc);
         lp.state_stride = ((16 * (size_t)lanes * ((size_t)l.n_slots + (size_t)H.nc)) + 255) & ~(size_t)255;
@@ -1018,7 +1042,42 @@ namespace b200
         lp.state = state_.p.get();
         launch_kernel(fn, ctas, threads, 0, s, lp, "layered kernel");
         release_state(s);
-        note_launch(fpc, threads, ctas, LDPC_B200_GLOBAL, tuning.precision, 0);
+        note_launch(fpc, threads, ctas, LDPC_B200_GLOBAL, q ? LDPC_B200_FIXED : tuning.precision, 0);
+    }
+
+    void Engine::quant_shape(int *lanes, int *threads, const void **fn, int *per_sm)
+    {
+        if (tuning.frames_per_cta != 0 && tuning.frames_per_cta != 16 && tuning.frames_per_cta != 32)
+            throw std::runtime_error("quantised decoding: frames_per_cta must be 0, 16 or 32");
+        *lanes = tuning.frames_per_cta == 16 ? 2 : 4;
+        *threads = tuning.threads_per_cta > 0 ? std::min(tuning.threads_per_cta, 512) : 256;
+        *fn = layered_kernel_q(*lanes);
+        CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, *fn, *threads, 0));
+    }
+
+    int64_t Engine::batch_wave(const decoder_param &dp, uint64_t n_frames, cudaStream_t s)
+    {
+        if (quantised())
+        {
+            int lanes, threads, per_sm;
+            const void *fn;
+            quant_shape(&lanes, &threads, &fn, &per_sm);
+            return (int64_t)sm_count_ * std::max(per_sm, 1) * lanes * 8;
+        }
+        maybe_autotune(alg_of(dp), dp, n_frames, s);
+        const Config c = choose(tuning.precision, alg_of(dp), ~0ull >> 1);
+        return (int64_t)c.ctas * c.fpc;
+    }
+
+    void Engine::set_quant(const ldpc_b200_quant *q)
+    {
+        if (!q || q->ch_bits == 0) { quant = ldpc_b200_quant{}; return; }
+        if (!(q->msg_bits >= 2 && q->msg_bits <= q->post_bits && q->post_bits <= 16 && q->ch_bits >= 2 && q->ch_bits <= q->post_bits))
+            throw std::runtime_error("quantisation: bit widths must satisfy 2 <= msg_bits <= post_bits <= 16 and 2 <= ch_bits <= post_bits");
+        if (q->offset < 0 || q->offset >= (1 << (q->msg_bits - 1)) - 1) throw std::runtime_error("quantisation: offset must satisfy 0 <= offset < 2^(msg_bits-1) - 1");
+        if (q->scale8 < 1 || q->scale8 > 8) throw std::runtime_error("quantisation: scale8 must be 1 .. 8");
+        if (!(q->step > 0) || !std::isfinite(q->step)) throw std::runtime_error("quantisation: step must be a finite value > 0");
+        quant = *q;
     }
 
     void Engine::launch_bec(const decoder_param &dp, const FrameSource &src, const FrameSink &sink, uint64_t n_frames, cudaStream_t s)
@@ -1188,6 +1247,7 @@ namespace b200
     {
         ensure_cuda();
         if (channel_kind(channel) == SRC_BEC) return (uint64_t)sm_count_ * 8 * 32; // bit-sliced kernel: up to 8 words of 32 frames per CTA
+        if (quantised()) return (uint64_t)batch_wave(dp, 0, stream_.get());
         const Config c = choose(tuning.precision, alg_of(dp), ~0ull >> 1);
         return (uint64_t)c.ctas * c.fpc;
     }
@@ -1246,9 +1306,7 @@ namespace b200
         // per launch, and a short pipeline fill
         int64_t chunk = std::max<int64_t>((int64_t)((32ull << 20) / (nc * esz)), 1), wave = 1;
         {
-            maybe_autotune(alg_of(dp), dp, (uint64_t)n, sk);
-            const Config c = choose(tuning.precision, alg_of(dp), ~0ull >> 1);
-            wave = (int64_t)c.ctas * c.fpc;
+            wave = batch_wave(dp, (uint64_t)n, sk);
             chunk = std::max<int64_t>(wave, chunk / wave * wave);
         }
         chunk = std::min<int64_t>(n, chunk);
@@ -1583,9 +1641,7 @@ namespace b200
         int64_t chunk = std::max<int64_t>((int64_t)((32ull << 20) / (nc * (bec ? 1 : sizeof(double)))), 1);
         if (!bec)
         {
-            maybe_autotune(alg_of(dp), dp, (uint64_t)n, s);
-            const Config c = choose(tuning.precision, alg_of(dp), ~0ull >> 1);
-            const int64_t wave = (int64_t)c.ctas * c.fpc;
+            const int64_t wave = batch_wave(dp, (uint64_t)n, s);
             chunk = std::max<int64_t>(wave, chunk / wave * wave);
         }
         chunk = std::min<int64_t>(chunk, n);

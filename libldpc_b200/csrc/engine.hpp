@@ -130,6 +130,11 @@ namespace b200
         }
         int fading_L = 1;
 
+        // fixed-point layered min-sum (DESIGN.md §3.7): ch_bits = 0 is off; set_quant validates and keeps the old setting on failure
+        void set_quant(const ldpc_b200_quant *q);
+        ldpc_b200_quant quant{};
+        bool quantised() const { return quant.ch_bits > 0; }
+
         // layered schedule: the layering in use (empty = built-in first-fit layering, made on first use)
         void set_layers(std::vector<std::vector<int>> layers);
         const std::vector<std::vector<int>> &layers();
@@ -164,6 +169,10 @@ namespace b200
                           const std::function<bool()> &eligible = nullptr);
         float time_ms(CUstream_st *s, const std::function<void()> &work); // device time of `work` on s (ev0_ .. ev1_; blocking)
         void maybe_autotune(int alg, const decoder_param &dp, uint64_t n_frames, CUstream_st *s);
+        // frames of one full wave of the persistent grid for a batch job of this decoder type (runs the shape trial first where it applies)
+        int64_t batch_wave(const decoder_param &dp, uint64_t n_frames, CUstream_st *s);
+        // the fixed-point layered kernel's shape under the current tuning: lanes per node, threads, the kernel, CTAs per SM
+        void quant_shape(int *lanes, int *threads, const void **fn, int *per_sm);
         // outcomes of the shape trials are remembered across processes: $LDPC_B200_TUNE_CACHE (a directory; "off" disables) or
         // ~/.cache/libldpc_b200, one small text file per (code, device)
         std::string tune_cache_file();

@@ -15,4 +15,10 @@ namespace b200
         if (lanes != 2 && lanes != 4) throw std::runtime_error("layered schedule: lanes per node must be 2 or 4");
         return kernels[f32][alg == ALG_BP][lanes == 4];
     }
+
+    const void *layered_kernel_q(int lanes)
+    {
+        if (lanes != 2 && lanes != 4) throw std::runtime_error("layered schedule: lanes per node must be 2 or 4");
+        return lanes == 4 ? (const void *)lay_kernel<int16_t, ALG_MS, 4> : (const void *)lay_kernel<int16_t, ALG_MS, 2>;
+    }
 } // namespace b200

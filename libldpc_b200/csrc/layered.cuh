@@ -15,6 +15,8 @@
 // LANES*VEC frames starts and retires together; converged lanes are frozen by masked stores).  Global residency only (the mode
 // is for quasi-cyclic codes of the 5G NR kind, whose state does not fit shared memory).
 #pragma once
+#include <type_traits>
+
 #include "tile4.cuh"
 
 namespace b200
@@ -42,6 +44,30 @@ namespace b200
         unsigned long long err_cap;
         unsigned char *state;
         size_t state_stride;
+        // fixed-point decoder (T = int16_t, DESIGN.md §3.7); appended so that the floating-point instantiations keep their offsets
+        double q_step;                       // LLR of one LSB
+        int q_ch_max, q_msg_max, q_post_max; // M(q) = 2^(q-1) - 1 of the channel, message and posterior widths
+        int q_offset, q_scale8;              // check output max(floor(m * scale8 / 8) - offset, 0)
+    };
+
+    // 16-byte vectors of 8 frame lanes of the fixed-point state
+    template <> struct __align__(16) Vec<int16_t> { static constexpr int N = 8; int16_t e[8]; };
+
+    // decoder state <-> fp64 LLR: the identity for double and float; for int16_t the quantiser clamp(round(L / step), -M(Qc), M(Qc))
+    // (division correctly rounded, round half away from zero) and, for llr_out, P * step correctly rounded
+    template <typename T> struct LayState
+    {
+        static __device__ __forceinline__ T in(double x, const LayParams &) { return (T)x; }
+        static __device__ __forceinline__ double out(T v, const LayParams &) { return (double)v; }
+    };
+    template <> struct LayState<int16_t>
+    {
+        static __device__ __forceinline__ int16_t in(double x, const LayParams &p)
+        {
+            const double m = (double)p.q_ch_max;
+            return (int16_t)(int)fmin(fmax(round(__ddiv_rn(x, p.q_step)), -m), m);
+        }
+        static __device__ __forceinline__ double out(int16_t v, const LayParams &p) { return __dmul_rn((double)v, p.q_step); }
     };
 
     // One check of degree `deg`: thread (node j, vector sub).  slot0 = first slot of the node (slot of edge k = slot0 + k * NPW).
@@ -209,6 +235,79 @@ namespace b200
         }
     }
 
+    // Fixed-point min-sum check of degree `deg` (the int16_t state of DESIGN.md §3.7; arguments as cn_lay).  int32 arithmetic:
+    // v = sat_Qp(P - c2v_old); magnitude of the others min(|v|, M(Qm)) (the running minima start at M(Qm)), sign product of the
+    // others (0 is positive); c2v = sign * max(floor(m * a / 8) - beta, 0); P = sat_Qp(v + c2v).
+    template <int LANES>
+    __device__ __forceinline__ void cn_lay_q(unsigned char *out_sub, unsigned char *c2v_sub, const uint32_t *__restrict__ idx, uint32_t slot0, int deg,
+                                             uint32_t fz, uint32_t live, const LayParams &p)
+    {
+        typedef Vec<int16_t> V;
+        constexpr int VEC = V::N, NPW = 32 / LANES, RS = 16 * LANES;
+        constexpr uint32_t VMASK = (1u << VEC) - 1u;
+        const int pm = p.q_post_max;
+        auto load_v = [&](int k, uint32_t &eo, int (&v)[VEC])
+        {
+            const uint32_t s = slot0 + (uint32_t)k * NPW;
+            eo = __ldg(idx + s);
+            const V o = *reinterpret_cast<const V *>(out_sub + eo);
+            const V c = *reinterpret_cast<const V *>(c2v_sub + (size_t)s * RS);
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) v[e] = min(max((int)o.e[e] - (((fz >> e) & 1u) ? 0 : (int)c.e[e]), -pm), pm);
+        };
+        int m1[VEC], m2[VEC], arg[VEC];
+        unsigned long long smask[VEC];
+#pragma unroll
+        for (int e = 0; e < VEC; ++e) { m1[e] = p.q_msg_max; m2[e] = p.q_msg_max; arg[e] = 0; smask[e] = 0; }
+        for (int k = 0; k < deg; ++k)
+        {
+            uint32_t eo;
+            int v[VEC];
+            load_v(k, eo, v);
+#pragma unroll
+            for (int e = 0; e < VEC; ++e)
+            {
+                smask[e] |= (unsigned long long)(v[e] < 0) << k;
+                const int a = abs(v[e]);
+                const bool lt1 = a < m1[e], lt2 = a < m2[e];
+                m2[e] = lt1 ? m1[e] : (lt2 ? a : m2[e]);
+                arg[e] = lt1 ? k : arg[e];
+                m1[e] = lt1 ? a : m1[e];
+            }
+        }
+        for (int k = 0; k < deg; ++k)
+        {
+            uint32_t eo;
+            int v[VEC];
+            load_v(k, eo, v); // the same operands as in the first pass: the same value
+            V r, o;
+#pragma unroll
+            for (int e = 0; e < VEC; ++e)
+            {
+                const int mag = max((((k == arg[e]) ? m2[e] : m1[e]) * p.q_scale8 >> 3) - p.q_offset, 0);
+                const int c = ((__popcll(smask[e]) ^ (int)(smask[e] >> k)) & 1) ? -mag : mag;
+                r.e[e] = (int16_t)c;
+                o.e[e] = (int16_t)min(max(v[e] + c, -pm), pm);
+            }
+            const uint32_t s = slot0 + (uint32_t)k * NPW;
+            if (live == VMASK)
+            {
+                *reinterpret_cast<V *>(c2v_sub + (size_t)s * RS) = r;
+                *reinterpret_cast<V *>(out_sub + eo) = o;
+            }
+            else
+            {
+#pragma unroll
+                for (int e = 0; e < VEC; ++e)
+                    if ((live >> e) & 1u)
+                    {
+                        *reinterpret_cast<int16_t *>(c2v_sub + (size_t)s * RS + e * 2) = r.e[e];
+                        *reinterpret_cast<int16_t *>(out_sub + eo + e * 2) = o.e[e];
+                    }
+            }
+        }
+    }
+
     // parity of the hard decisions of one check's variables, per frame lane of the vector (decoder.h:47-64)
     template <typename T, int LANES>
     __device__ __forceinline__ uint32_t synd_lay(const unsigned char *out_sub, const uint32_t *__restrict__ idx, uint32_t slot0, int deg)
@@ -276,7 +375,7 @@ namespace b200
                 if (p.kind == SRC_LLR)
                 {
                     const double *src = p.llr_in + (size_t)(f0 + g) * p.nc;
-                    for (int i = tid; i < p.nc; i += nthreads) put(i, (T)src[i]);
+                    for (int i = tid; i < p.nc; i += nthreads) put(i, LayState<T>::in(src[i], p));
                     continue;
                 }
                 const unsigned long long frame = p.frame0 + f0 + g;
@@ -290,7 +389,7 @@ namespace b200
                         normal_pair(r.z, r.w, z[2], z[3]);
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
-                            if (q + k * nblk < p.nct) put(p.tx_var[q + k * nblk], (T)__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), 1.0), p.llr_scale));
+                            if (q + k * nblk < p.nct) put(p.tx_var[q + k * nblk], LayState<T>::in(__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), 1.0), p.llr_scale), p));
                     }
                     else if (p.kind == SRC_RAYLEIGH)
                     {
@@ -303,7 +402,7 @@ namespace b200
                             const int t = q + k * nblk;
                             if (t >= p.nct) continue;
                             const double h = rayleigh_coeff(p.seed, p.point, frame, p.coherence ? (uint32_t)(t / p.coherence) : 0u);
-                            put(p.tx_var[t], (T)__dmul_rn(__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), h), h), p.llr_scale));
+                            put(p.tx_var[t], LayState<T>::in(__dmul_rn(__dmul_rn(__dadd_rn(__dmul_rn((double)z[k], p.sigma), h), h), p.llr_scale), p));
                         }
                     }
                     else
@@ -311,12 +410,18 @@ namespace b200
                         const uint32_t w[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
-                            if (q + k * nblk < p.nct) put(p.tx_var[q + k * nblk], (T)((w[k] < p.thr) ? -p.delta : p.delta));
+                            if (q + k * nblk < p.nct) put(p.tx_var[q + k * nblk], LayState<T>::in((w[k] < p.thr) ? -p.delta : p.delta, p));
                     }
                 }
                 for (int i = tid; i < p.n_punct; i += nthreads) put(p.punct[i], T(0));
-                for (int i = tid; i < p.n_short; i += nthreads) put(p.shorten[i], (T)(p.kind == SRC_BSC ? p.delta : 99999.9));
+                for (int i = tid; i < p.n_short; i += nthreads) put(p.shorten[i], LayState<T>::in(p.kind == SRC_BSC ? p.delta : 99999.9, p));
             }
+            // The syndrome slots are cleared once per CTA above, and s_synd[(it + 1) & 1] after every iteration: a batch that ends at
+            // an odd iteration limit with lanes still decoding leaves its last slot set for the next batch of the CTA.
+            // The fixed-point decoder clears both slots for every batch; the floating-point ones keep their results until that
+            // is fixed on its own.
+            if constexpr (std::is_same<T, int16_t>::value)
+                if (tid < 2) s_synd[tid] = 0;
             __syncthreads();
 
             uint32_t live = valid;       // CTA-uniform: lanes still decoding
@@ -329,7 +434,10 @@ namespace b200
                 const uint32_t mylive = (live >> (sub * VEC)) & VMASK, fz = (it == 0) ? VMASK : 0u;
                 for (int l = 0; l < p.n_layers; ++l)
                 {
-                    for_tasks(l, [&](int deg, uint32_t slot0) { cn_lay<T, ALG, LANES>(out_sub, c2v_sub, p.idx, slot0, deg, fz, mylive, (T)p.ms_scale); });
+                    if constexpr (std::is_same<T, int16_t>::value)
+                        for_tasks(l, [&](int deg, uint32_t slot0) { cn_lay_q<LANES>(out_sub, c2v_sub, p.idx, slot0, deg, fz, mylive, p); });
+                    else
+                        for_tasks(l, [&](int deg, uint32_t slot0) { cn_lay<T, ALG, LANES>(out_sub, c2v_sub, p.idx, slot0, deg, fz, mylive, (T)p.ms_scale); });
                     __syncthreads(); // the next layer reads the posteriors this one wrote
                 }
                 executed += (unsigned long long)__popc(live);
@@ -364,7 +472,7 @@ namespace b200
                         for (int i = tid; i < p.nc; i += nthreads)
                         {
                             const T v = *reinterpret_cast<const T *>(src + (size_t)i * RS);
-                            if (p.llr_out) p.llr_out[o + i] = (double)v;
+                            if (p.llr_out) p.llr_out[o + i] = LayState<T>::out(v, p);
                             if (p.hard_out) p.hard_out[o + i] = (v <= T(0)) ? 1 : 0;
                         }
                     }
@@ -399,4 +507,6 @@ namespace b200
 
     // the layered kernel for (precision, algorithm, lanes per node: 2 or 4); layered.cu instantiates them
     const void *layered_kernel(bool f32, int alg, int lanes);
+    // the fixed-point (int16_t, min-sum) layered kernel, lanes per node 2 or 4 (16 or 32 frames per CTA)
+    const void *layered_kernel_q(int lanes);
 } // namespace b200

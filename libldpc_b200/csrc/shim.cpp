@@ -236,6 +236,22 @@ extern "C"
         });
     }
 
+    int ldpc_b200_set_quant(ldpc_b200_ctx *ctx, const ldpc_b200_quant *q)
+    {
+        return guarded([&] {
+            if (!ctx) throw std::runtime_error("null argument");
+            ctx->eng->set_quant(q);
+        });
+    }
+
+    int ldpc_b200_get_quant(const ldpc_b200_ctx *ctx, ldpc_b200_quant *q)
+    {
+        return guarded([&] {
+            if (!ctx || !q) throw std::runtime_error("null argument");
+            *q = ctx->eng->quant;
+        });
+    }
+
     int ldpc_b200_set_layers(ldpc_b200_ctx *ctx, int n_layers, const int *layer_ptr, const int *layer_check)
     {
         return guarded([&] {
