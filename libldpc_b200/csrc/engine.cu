@@ -788,7 +788,9 @@ namespace b200
 
     void Engine::maybe_autotune(int alg, const decoder_param &dp, uint64_t n_frames, cudaStream_t s)
     {
-        if (quantised()) return; // the fixed-point kernel has one shape: no trial, and nothing stored under a flooding key
+        // The trials time launch(), which serves the layered schedule (and the fixed-point decoder) with the layered kernel: its
+        // outcome would be stored, and cached on disk, as the flooding kernel's shape.  The layered kernel has no shape trial.
+        if (quantised() || tuning.schedule != LDPC_B200_FLOODING) return;
         tune_cache_load();
         const auto key = std::make_pair(tuning.precision, alg);
         if (in_autotune_ || n_frames < 20000 || tuning.frames_per_cta > 0 || tuning.threads_per_cta > 0 || tuned_.count(key) || pair_tuned_.count(key)) return;

@@ -416,12 +416,9 @@ namespace b200
                 for (int i = tid; i < p.n_punct; i += nthreads) put(p.punct[i], T(0));
                 for (int i = tid; i < p.n_short; i += nthreads) put(p.shorten[i], LayState<T>::in(p.kind == SRC_BSC ? p.delta : 99999.9, p));
             }
-            // The syndrome slots are cleared once per CTA above, and s_synd[(it + 1) & 1] after every iteration: a batch that ends at
-            // an odd iteration limit with lanes still decoding leaves its last slot set for the next batch of the CTA.
-            // The fixed-point decoder clears both slots for every batch; the floating-point ones keep their results until that
-            // is fixed on its own.
-            if constexpr (std::is_same<T, int16_t>::value)
-                if (tid < 2) s_synd[tid] = 0;
+            // Both syndrome slots start every batch cleared: a batch that ends at its iteration limit with lanes still decoding
+            // leaves its last slot set, and the next batch of the CTA must not OR those bits into its own iteration-0 test.
+            if (tid < 2) s_synd[tid] = 0;
             __syncthreads();
 
             uint32_t live = valid;       // CTA-uniform: lanes still decoding
