@@ -294,7 +294,8 @@ namespace b200
         static constexpr int VEC = V::N, CS = 512;
 
         // CSRC: the old c2v values come from shared/global memory (0, 2) or from the thread's TMEM mirror at
-        // columns tc + 4k (1, 3); 2 and 3 force the fresh frame lanes `fz` to +0; TMW: new values are also written to the mirror.
+        // columns tc + 4k (1, 3); 2 and 3 force the fresh frame lanes `fz` to +0; 4: every lane's old c2v is +0 (first check
+        // phase of a lock-step batch), so v2c = out and no c2v is read; TMW: new values are also written to the mirror.
         // nx: in = this node's index entries (byte offsets), out = those of the node at ip_next when `more`
         // (software prefetch: the load is in flight while this node is computed).
         // PAR: also return the syndrome bits (only early termination consumes them, decoder.cpp:66-72).
@@ -322,8 +323,8 @@ namespace b200
                     const V o = VAcc<SMEM, T, 0>::ld(out_sub + eo[k.value]);
                     V c;
                     if constexpr (CSRC == 1 || CSRC == 3) { c = TmAcc<T>::ld(tc + 4 * k.value); tm_wait_ld(); }
-                    else c = VAcc<SMEM, T, k.value * CS>::ld(c2v0);
-                    if constexpr (CSRC >= 2)
+                    else if constexpr (CSRC != 4) c = VAcc<SMEM, T, k.value * CS>::ld(c2v0);
+                    if constexpr (CSRC == 2 || CSRC == 3)
                     {
 #pragma unroll
                         for (int e = 0; e < VEC; ++e) c.e[e] = ((fz >> e) & 1u) ? T(0) : c.e[e];
@@ -331,7 +332,8 @@ namespace b200
 #pragma unroll
                     for (int e = 0; e < VEC; ++e)
                     {
-                        const T v = o.e[e] - c.e[e]; // == the reference's stored v2c (decoder.cpp:62); LLRin on a fresh frame (:18)
+                        T v = o.e[e]; // out - (+0) == out for every out, -0 included
+                        if constexpr (CSRC != 4) v = o.e[e] - c.e[e]; // == the reference's stored v2c (decoder.cpp:62); LLRin on a fresh frame (:18)
                         if constexpr (PAR) par[e] ^= (o.e[e] <= T(0));
                         sm[e] |= (Num<T>::hi(v) >> 31) << k.value;
                         const bool lt1 = Num<T>::abs(v) < Num<T>::abs(m1[e]), lt2 = Num<T>::abs(v) < Num<T>::abs(m2[e]);
@@ -356,10 +358,10 @@ namespace b200
                 V v[D], r[D], c[D];
                 static_for<D>([&](auto k) {
                     if constexpr (CSRC == 1 || CSRC == 3) c[k.value] = TmAcc<T>::ld(tc + 4 * k.value);
-                    else c[k.value] = VAcc<SMEM, T, k.value * CS>::ld(c2v0);
+                    else if constexpr (CSRC != 4) c[k.value] = VAcc<SMEM, T, k.value * CS>::ld(c2v0);
                 });
                 if constexpr (CSRC == 1 || CSRC == 3) tm_wait_ld();
-                if constexpr (CSRC >= 2)
+                if constexpr (CSRC == 2 || CSRC == 3)
                 {
 #pragma unroll
                     for (int k = 0; k < D; ++k)
@@ -373,7 +375,8 @@ namespace b200
 #pragma unroll
                     for (int e = 0; e < VEC; ++e)
                     {
-                        v[k.value].e[e] = o.e[e] - c[k.value].e[e];
+                        if constexpr (CSRC == 4) v[k.value].e[e] = o.e[e];
+                        else v[k.value].e[e] = o.e[e] - c[k.value].e[e];
                         if constexpr (PAR) par[e] ^= (o.e[e] <= T(0));
                     }
                 });
@@ -1162,52 +1165,36 @@ namespace b200
         __shared__ long long s_pt[2][32]; // work-end time stamps of the warps (a barrier releases at their maximum)
         long long pt_vcyc[3] = {0, 0, 0}, pt_vtask[3] = {0, 0, 0};
 #endif
-        // The loop advances by HALF iterations (even h: check phase, odd h: variable phase) so that the retire / refill event
-        // has exactly ONE call site, at the top of a half: a frame lane found finished is recorded as pending and handled when
-        // the next half begins.  (The event is ~1 k instructions of cold code; inlined at three sites it no longer shared the
-        // 32 KB instruction cache with the decode loop and every event paid for instruction fetches from L2.)
+        // state of the half-iteration loop (ET kernels, below)
         uint32_t pend_mask = ALL, pend_synd = 0, pend_started = 0; // the initial fill is the first event
         bool pend_skip = false, pend_first = true, pend_clear = false;
         int par_i = 1; // parity of the iteration in progress (double-buffered control words); the first check half makes it 0
 #ifdef B200_PHASE_TIMING
         long long pt1 = 0, pt2 = 0;
 #endif
-        for (uint32_t h = 0;; ++h)
+        // ---- check-node phase (+ syndrome of the previous iteration's decisions, ORed into `bad`: ET kernels) -----
+        uint32_t bad = 0;
+        auto cn_phase = [&](auto csrc)
         {
-            if (pend_mask)
+            constexpr int CSRC = decltype(csrc)::value;
+            const uint32_t fz = (fresh >> (sub * VEC)) & VMASK;
+            uint32_t tc = tm_w;
+            uint4 sg_next = WAcc<SMEM, 0>::ld4(cn_seg_w);
+            for (P sp = cn_seg_w;;)
             {
-                retire_and_refill(pend_mask, pend_synd, pend_started, pend_skip, pend_first);
-                if (pend_clear && warp == 0 && lane == 0) s_ctrl[par_i ^ 1].x &= ~pend_mask; // consumed (everyone read it before the event's barriers)
-                pend_mask = 0; pend_first = false; pend_clear = false;
-            }
-            if (!(h & 1u))
-            {
-            if (!active) break; // CTA-uniform
-            par_i ^= 1;
-
-            // ---- check-node phase (+ syndrome of the previous iteration's decisions) ----------
-            uint32_t bad = 0;
-            auto cn_phase = [&](auto csrc)
-            {
-                constexpr int CSRC = decltype(csrc)::value;
-                const uint32_t fz = (fresh >> (sub * VEC)) & VMASK;
-                uint32_t tc = tm_w;
-                uint4 sg_next = WAcc<SMEM, 0>::ld4(cn_seg_w);
-                for (P sp = cn_seg_w;;)
-                {
 #ifdef B200_PHASE_TIMING
-                    const long long ph0 = clock64();
+                const long long ph0 = clock64();
 #endif
-                    const uint4 sg = SMEM ? uniform4(sg_next) : sg_next;
-                    if (sg.x == 0) break;
-                    sp += 16;
-                    sg_next = WAcc<SMEM, 0>::ld4(sp); // the next descriptor (or the terminator) is in flight while this segment runs
-                    // threads of nodes missing from a ragged task run along on padded slots / zero index entries
-                    const int deg = (int)(sg.x & 0xFFu);
-                    const uint32_t keep = (j < (int)((sg.x >> 8) & 0xFFu)) ? 0xFFFFFFFFu : 0u;
-                    int nt = (int)(sg.x >> 16);
-                    P c2v0 = c2v_lane + sg.y;
-                    const P ib = cn_idx + sg.z;
+                const uint4 sg = SMEM ? uniform4(sg_next) : sg_next;
+                if (sg.x == 0) break;
+                sp += 16;
+                sg_next = WAcc<SMEM, 0>::ld4(sp); // the next descriptor (or the terminator) is in flight while this segment runs
+                // threads of nodes missing from a ragged task run along on padded slots / zero index entries
+                const int deg = (int)(sg.x & 0xFFu);
+                const uint32_t keep = (j < (int)((sg.x >> 8) & 0xFFu)) ? 0xFFFFFFFFu : 0u;
+                int nt = (int)(sg.x >> 16);
+                P c2v0 = c2v_lane + sg.y;
+                const P ib = cn_idx + sg.z;
 #ifdef B200_PHASE_TIMING
 #define B200_PT_HDR pt_hdr += clock64() - ph0; pt_nseg += 1; pt_ntask += nt;
 #else
@@ -1233,32 +1220,211 @@ namespace b200
         }                                                                                                    \
         break;                                                                                               \
     }
-                    switch (deg) // warp-uniform
+                switch (deg) // warp-uniform
+                {
+                    B200_CN_CASE(2)
+                    B200_CN_CASE(3)
+                    B200_CN_CASE(4)
+                    B200_CN_CASE(5)
+                    B200_CN_CASE(6)
+                    B200_CN_CASE(7)
+                    B200_CN_CASE(8)
+                default: // not mirrored: always served from shared / global memory
+                {
+                    const int st = idx_stride_of(deg, ISZ);
+                    P ip = ib + j * 16;
+                    for (; nt > 0; --nt)
                     {
-                        B200_CN_CASE(2)
-                        B200_CN_CASE(3)
-                        B200_CN_CASE(4)
-                        B200_CN_CASE(5)
-                        B200_CN_CASE(6)
-                        B200_CN_CASE(7)
-                        B200_CN_CASE(8)
-                    default: // not mirrored: always served from shared / global memory
+                        bad |= cn4_any<T, IdxT, SMEM, LANES, ALG>(out_sub, c2v0, ip, deg, CSRC == 4 ? VMASK : CSRC >= 2 ? fz : 0u) & keep;
+                        c2v0 += deg * 512;
+                        ip += NPW * st;
+                    }
+                    break;
+                }
+                }
+#undef B200_CN_CASE
+            }
+            if constexpr (TM) tm_wait_st();
+        };
+        // ---- variable-node phase: posterior (hard decision = its sign, taken where it is consumed); frame lanes outside
+        //      `mylive` (bits of this thread's vector) keep their posterior.  The lock-step loop never clears a bit. ----
+        uint32_t mylive = VMASK;
+        auto vn_phase = [&](auto lsrc)
+        {
+            constexpr int LSRC = decltype(lsrc)::value;
+            uint32_t tl = tm_w + p.tm_vn_off;
+            uint4 sg_next = WAcc<SMEM, 0>::ld4(vn_seg_w);
+            for (P sp = vn_seg_w;;)
+            {
+                const uint4 sg = SMEM ? uniform4(sg_next) : sg_next;
+                if (sg.x == 0) break;
+                sp += 16;
+                sg_next = WAcc<SMEM, 0>::ld4(sp);
+                const int deg = (int)(sg.x & 0xFFu);
+                int nt = (int)(sg.x >> 16);
+#ifdef B200_PHASE_TIMING
+                const long long vs0 = clock64();
+                const int vcls = deg == 1 ? 0 : deg == 2 ? 1 : 2;
+                pt_vtask[vcls] += nt;
+#endif
+                P lp = llr_lane + sg.y, op = out_lane + sg.y;
+                const P ib = vn_idx + sg.z;
+                auto channel_llr = [&]() -> V // decoder.cpp:50
+                {
+                    V a;
+                    if constexpr (LSRC == 1) { a = TmAcc<T>::ld(tl); tm_wait_ld(); }
+                    else
+                    {
+                        a = VAcc<SMEM, T, 0>::ld(lp);
+                        if constexpr (TM) TmAcc<T>::st(tl, a);
+                    }
+                    return a;
+                };
+                auto finish = [&](const V &acc)
+                {
+                    if (mylive == VMASK) VAcc<SMEM, T, 0>::st(op, acc);
+                    else
+                    {
+#pragma unroll
+                        for (int e = 0; e < VEC; ++e)
+                            if ((mylive >> e) & 1u) Acc<SMEM, T, 0>::st(op + e * TS, acc.e[e]);
+                    }
+                    lp += 512;
+                    op += 512;
+                    if constexpr (TM) tl += 4;
+                };
+#define B200_VN_CASE(D)                                                                                      \
+    case D:                                                                                                  \
+    {                                                                                                        \
+        constexpr int ST = idx_stride_of(D, ISZ);                                                            \
+        P ip = ib + j * (ST < 16 ? ST : 16);                                                                 \
+        uint32_t nx[D];                                                                                      \
+        IdxLoad<SMEM, IdxT, LANES, D>::load(ip, nx);                                                         \
+        _Pragma("unroll 1") for (; nt > 0; --nt)                                                             \
+        {                                                                                                    \
+            ip += NPW * ST;                                                                                  \
+            finish(Vn4<T, IdxT, SMEM, LANES, D>::run(c2v_sub, nx, ip, nt > 1, channel_llr()));               \
+        }                                                                                                    \
+        break;                                                                                               \
+    }
+                switch (deg)
+                {
+                case 0:
+                    for (; nt > 0; --nt) finish(channel_llr());
+                    break;
+                    B200_VN_CASE(1)
+                    B200_VN_CASE(2)
+                    B200_VN_CASE(3)
+                    B200_VN_CASE(4)
+                    B200_VN_CASE(5)
+                    B200_VN_CASE(6)
+                    B200_VN_CASE(7)
+                    B200_VN_CASE(8)
+                default:
+                {
+                    auto generic = [&]()
                     {
                         const int st = idx_stride_of(deg, ISZ);
                         P ip = ib + j * 16;
                         for (; nt > 0; --nt)
                         {
-                            bad |= cn4_any<T, IdxT, SMEM, LANES, ALG>(out_sub, c2v0, ip, deg, CSRC >= 2 ? fz : 0u) & keep;
-                            c2v0 += deg * 512;
+                            finish(vn4_any<T, IdxT, SMEM, LANES>(c2v_sub, ip, deg, channel_llr()));
                             ip += NPW * st;
                         }
-                        break;
+                    };
+                    if constexpr (SMEM)
+                    { // the 128-register kernels also unroll degrees 9..16: every gather of the node is in flight before the
+                      // (strictly ordered) additions start
+                        switch (deg)
+                        {
+                            B200_VN_CASE(9)
+                            B200_VN_CASE(10)
+                            B200_VN_CASE(11)
+                            B200_VN_CASE(12)
+                            B200_VN_CASE(13)
+                            B200_VN_CASE(14)
+                            B200_VN_CASE(15)
+                            B200_VN_CASE(16)
+                        default: generic(); break;
+                        }
                     }
-                    }
-#undef B200_CN_CASE
+                    else generic();
+                    break;
                 }
-                if constexpr (TM) tm_wait_st();
-            };
+                }
+#undef B200_VN_CASE
+#ifdef B200_PHASE_TIMING
+                pt_vcyc[vcls] += clock64() - vs0;
+#endif
+            }
+            if constexpr (TM && LSRC == 0) tm_wait_st();
+        };
+
+        // The retire / refill event has exactly ONE call site per kernel.  (The event is ~1 k instructions of cold code; inlined at
+        // three sites it no longer shared the 32 KB instruction cache with the decode loop and every event paid for instruction
+        // fetches from L2.)
+        if constexpr (!ET)
+        {
+            // Without early termination every frame lane of the CTA is filled by the same event and reaches max_iter in the same
+            // iteration, so the CTA decodes in lock-step batches: fill, max_iter x (check phase, barrier, variable phase,
+            // barrier), retire -- the event's call site is the top of a batch and nothing is decided per half iteration.  In a
+            // ragged last batch the lanes without a frame compute on whatever their slots hold (arithmetic on shared memory and
+            // TMEM only, nothing can fault); nothing reads those lanes.
+            for (bool first = true;; first = false)
+            {
+                retire_and_refill(first ? ALL : active, 0u, 0u, false, first);
+                if (!active) break; // CTA-uniform
+                for (int i = 0; i < p.max_iter; ++i)
+                {
+                    // first iteration of a batch: every old c2v is +0 and the channel LLRs sit in shared memory only (the variable
+                    // phase refreshes their mirror); the later ones read the mirror
+                    if (i == 0) cn_phase(std::integral_constant<int, 4>{});
+                    else cn_phase(std::integral_constant<int, 1>{});
+#ifdef B200_PHASE_TIMING
+                    pt1 = clock64();
+                    if (lane == 0) s_pt[0][warp] = pt1;
+#endif
+                    __syncthreads(); // B
+#ifdef B200_PHASE_TIMING
+                    pt2 = 0;
+                    for (int w = 0; w < warps; ++w) pt2 = max(pt2, s_pt[0][w]);
+#endif
+                    if (i == 0) vn_phase(std::integral_constant<int, 0>{});
+                    else vn_phase(std::integral_constant<int, 1>{});
+#ifdef B200_PHASE_TIMING
+                    const long long pt3 = clock64();
+                    if (lane == 0) s_pt[1][warp] = pt3;
+#endif
+                    __syncthreads(); // A
+#ifdef B200_PHASE_TIMING
+                    long long pt4 = 0;
+                    for (int w = 0; w < warps; ++w) pt4 = max(pt4, s_pt[1][w]);
+                    if (pt_rel) { pt_cn += pt1 - pt_rel; pt_wb += pt2 - pt1; pt_vn += pt3 - pt2; pt_wa += pt4 - pt3; ++pt_n; }
+                    pt_rel = pt4;
+#endif
+                }
+                it = p.max_iter;
+            }
+        }
+        else
+        {
+        // The loop advances by HALF iterations (even h: check phase, odd h: variable phase) so that the event can be called at
+        // the top of a half: a frame lane found finished is recorded as pending and handled when the next half begins.
+        for (uint32_t h = 0;; ++h)
+        {
+            if (pend_mask)
+            {
+                retire_and_refill(pend_mask, pend_synd, pend_started, pend_skip, pend_first);
+                if (pend_clear && warp == 0 && lane == 0) s_ctrl[par_i ^ 1].x &= ~pend_mask; // consumed (everyone read it before the event's barriers)
+                pend_mask = 0; pend_first = false; pend_clear = false;
+            }
+            if (!(h & 1u))
+            {
+            if (!active) break; // CTA-uniform
+            par_i ^= 1;
+
+            // ---- check-node phase (+ syndrome of the previous iteration's decisions) ----------
+            bad = 0;
             // right after a refill the fresh lanes' old c2v is forced to +0 (the mirror itself never goes stale: the check
             // phase is the only writer of c2v and writes through)
             if (!cn_stale) cn_phase(std::integral_constant<int, TM ? 1 : 0>{});
@@ -1304,117 +1470,7 @@ namespace b200
             }
 
             // ---- variable-node phase: posterior (hard decision = its sign, taken where it is consumed) ----
-            const uint32_t mylive = (live >> (sub * VEC)) & VMASK;
-            auto vn_phase = [&](auto lsrc)
-            {
-                constexpr int LSRC = decltype(lsrc)::value;
-                uint32_t tl = tm_w + p.tm_vn_off;
-                uint4 sg_next = WAcc<SMEM, 0>::ld4(vn_seg_w);
-                for (P sp = vn_seg_w;;)
-                {
-                    const uint4 sg = SMEM ? uniform4(sg_next) : sg_next;
-                    if (sg.x == 0) break;
-                    sp += 16;
-                    sg_next = WAcc<SMEM, 0>::ld4(sp);
-                    const int deg = (int)(sg.x & 0xFFu);
-                    int nt = (int)(sg.x >> 16);
-#ifdef B200_PHASE_TIMING
-                    const long long vs0 = clock64();
-                    const int vcls = deg == 1 ? 0 : deg == 2 ? 1 : 2;
-                    pt_vtask[vcls] += nt;
-#endif
-                    P lp = llr_lane + sg.y, op = out_lane + sg.y;
-                    const P ib = vn_idx + sg.z;
-                    auto channel_llr = [&]() -> V // decoder.cpp:50
-                    {
-                        V a;
-                        if constexpr (LSRC == 1) { a = TmAcc<T>::ld(tl); tm_wait_ld(); }
-                        else
-                        {
-                            a = VAcc<SMEM, T, 0>::ld(lp);
-                            if constexpr (TM) TmAcc<T>::st(tl, a);
-                        }
-                        return a;
-                    };
-                    auto finish = [&](const V &acc)
-                    {
-                        if (mylive == VMASK) VAcc<SMEM, T, 0>::st(op, acc);
-                        else
-                        {
-#pragma unroll
-                            for (int e = 0; e < VEC; ++e)
-                                if ((mylive >> e) & 1u) Acc<SMEM, T, 0>::st(op + e * TS, acc.e[e]);
-                        }
-                        lp += 512;
-                        op += 512;
-                        if constexpr (TM) tl += 4;
-                    };
-#define B200_VN_CASE(D)                                                                                      \
-    case D:                                                                                                  \
-    {                                                                                                        \
-        constexpr int ST = idx_stride_of(D, ISZ);                                                            \
-        P ip = ib + j * (ST < 16 ? ST : 16);                                                                 \
-        uint32_t nx[D];                                                                                      \
-        IdxLoad<SMEM, IdxT, LANES, D>::load(ip, nx);                                                         \
-        _Pragma("unroll 1") for (; nt > 0; --nt)                                                             \
-        {                                                                                                    \
-            ip += NPW * ST;                                                                                  \
-            finish(Vn4<T, IdxT, SMEM, LANES, D>::run(c2v_sub, nx, ip, nt > 1, channel_llr()));               \
-        }                                                                                                    \
-        break;                                                                                               \
-    }
-                    switch (deg)
-                    {
-                    case 0:
-                        for (; nt > 0; --nt) finish(channel_llr());
-                        break;
-                        B200_VN_CASE(1)
-                        B200_VN_CASE(2)
-                        B200_VN_CASE(3)
-                        B200_VN_CASE(4)
-                        B200_VN_CASE(5)
-                        B200_VN_CASE(6)
-                        B200_VN_CASE(7)
-                        B200_VN_CASE(8)
-                    default:
-                    {
-                        auto generic = [&]()
-                        {
-                            const int st = idx_stride_of(deg, ISZ);
-                            P ip = ib + j * 16;
-                            for (; nt > 0; --nt)
-                            {
-                                finish(vn4_any<T, IdxT, SMEM, LANES>(c2v_sub, ip, deg, channel_llr()));
-                                ip += NPW * st;
-                            }
-                        };
-                        if constexpr (SMEM)
-                        { // the 128-register kernels also unroll degrees 9..16: every gather of the node is in flight before the
-                          // (strictly ordered) additions start
-                            switch (deg)
-                            {
-                                B200_VN_CASE(9)
-                                B200_VN_CASE(10)
-                                B200_VN_CASE(11)
-                                B200_VN_CASE(12)
-                                B200_VN_CASE(13)
-                                B200_VN_CASE(14)
-                                B200_VN_CASE(15)
-                                B200_VN_CASE(16)
-                            default: generic(); break;
-                            }
-                        }
-                        else generic();
-                        break;
-                    }
-                    }
-#undef B200_VN_CASE
-#ifdef B200_PHASE_TIMING
-                    pt_vcyc[vcls] += clock64() - vs0;
-#endif
-                }
-                if constexpr (TM && LSRC == 0) tm_wait_st();
-            };
+            mylive = (live >> (sub * VEC)) & VMASK;
             if (live)
             {
                 if (TM && !vn_stale) vn_phase(std::integral_constant<int, TM ? 1 : 0>{});
@@ -1441,6 +1497,7 @@ namespace b200
                 if (lim) { pend_mask = lim; pend_synd = 0; pend_started = 0; pend_skip = false; pend_clear = true; }
             }
             }
+        }
         }
 #ifdef B200_PHASE_TIMING
         if (blockIdx.x == 0 && lane == 0)
