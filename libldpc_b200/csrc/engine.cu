@@ -345,6 +345,8 @@ namespace b200
         // share a TMEM lane partition (warp % 4) lie side by side in the 512 columns.
         c.tm = false;
         c.tm_alloc_cols = c.tm_cols_per_warp = c.tm_vn_off = 0;
+        c.lockstep = false;
+        c.tm_idx_off = 0;
         c.wide = false;
         if (c.residency == LDPC_B200_GLOBAL)
         {
@@ -357,32 +359,45 @@ namespace b200
         }
         if (c.residency == LDPC_B200_SMEM && tuning.tmem == 0)
         {
-            uint32_t cn_max = 0, vn_max = 0;
+            // the lock-step kernel also keeps every gather address of a warp's tasks in its window (ls_idx_cols per task)
+            uint32_t cn_max = 0, vn_max = 0, idx_max = 0;
             for (int w = 0; w < l.warps; ++w)
             {
-                uint32_t cn = 0, vn = 0;
+                uint32_t cn = 0, vn = 0, idx = 0;
                 for (int sgi = 0; sgi < l.cn_max_segs; ++sgi)
                 {
                     const uint32_t d = l.cn_seg[4 * ((size_t)w * l.cn_max_segs + sgi)];
                     if (!d) break;
                     cn += (d & 0xFFu) * (d >> 16);
+                    idx += (uint32_t)ls_idx_cols(true, (int)(d & 0xFFu)) * (d >> 16);
                 }
                 for (int sgi = 0; sgi < l.vn_max_segs; ++sgi)
                 {
                     const uint32_t d = l.vn_seg[4 * ((size_t)w * l.vn_max_segs + sgi)];
                     if (!d) break;
                     vn += d >> 16;
+                    idx += (uint32_t)ls_idx_cols(false, (int)(d & 0xFFu)) * (d >> 16);
                 }
                 cn_max = std::max(cn_max, cn);
                 vn_max = std::max(vn_max, vn);
+                idx_max = std::max(idx_max, idx);
             }
-            const uint32_t per_warp = 4 * (cn_max + vn_max), total = per_warp * (uint32_t)((l.warps + 3) / 4);
+            const uint32_t windows = (uint32_t)((l.warps + 3) / 4), per_warp = 4 * (cn_max + vn_max), total = per_warp * windows;
             if (total <= 512)
             {
                 uint32_t cols = 32;
                 while (cols < total) cols <<= 1;
                 c.tm = true;
                 c.tm_alloc_cols = cols; c.tm_cols_per_warp = per_warp; c.tm_vn_off = 4 * cn_max;
+                // Fixed iterations run the lock-step kernel when the gather addresses fit the mirror's allocation (the shape, the
+                // occupancy and the TMEM a CTA holds stay as they are) and the descriptors fit K4Params::ls_seg; otherwise the
+                // early-termination kernel runs them with early termination off.
+                if ((per_warp + idx_max) * windows <= cols && (size_t)l.warps * (size_t)(l.cn_max_segs + l.vn_max_segs) <= (size_t)K4_LS_SEGS)
+                {
+                    c.lockstep = true;
+                    c.tm_idx_off = per_warp;
+                    c.tm_cols_per_warp = per_warp + idx_max;
+                }
             }
         }
         c.idx16 = l.isz == 2;
@@ -441,7 +456,7 @@ namespace b200
     const void *Engine::tile_fn(const Config &c, bool et)
     {
         const bool smem = c.residency == LDPC_B200_SMEM;
-        const void *fn = tile_kernel(c.precision == LDPC_B200_F32, c.alg, c.lanes, smem, c.tm, et, c.wide, c.idx16);
+        const void *fn = tile_kernel(c.precision == LDPC_B200_F32, c.alg, c.lanes, smem, c.tm, et || !c.lockstep, c.wide, c.idx16);
         set_smem_attributes(fn, TILE_SMEM_OPTIN, smem);
         return fn;
     }
@@ -707,6 +722,23 @@ namespace b200
             kp.state = state_.p.get();
         }
         kp.tm_alloc_cols = c.tm_alloc_cols; kp.tm_cols_per_warp = c.tm_cols_per_warp; kp.tm_vn_off = c.tm_vn_off;
+        if (c.lockstep)
+        { // the segment descriptors travel in the parameters: check lists, then variable lists (tile4.cuh K4Params::ls_seg)
+            kp.tm_idx_off = c.tm_idx_off;
+            std::copy(l.cn_seg.begin(), l.cn_seg.end(), kp.ls_seg);
+            std::copy(l.vn_seg.begin(), l.vn_seg.end(), kp.ls_seg + l.cn_seg.size());
+            for (int w = 0; w < l.warps; ++w)
+            { // where the warp's variable-side addresses start: after its check-side ones
+                uint32_t cols = 0;
+                for (int sgi = 0; sgi < l.cn_max_segs; ++sgi)
+                {
+                    const uint32_t d = l.cn_seg[4 * ((size_t)w * l.cn_max_segs + sgi)];
+                    if (!d) break;
+                    cols += (uint32_t)ls_idx_cols(true, (int)(d & 0xFFu)) * (d >> 16);
+                }
+                kp.ls_seg[l.cn_seg.size() + 4 * (size_t)w * l.vn_max_segs + 3] = cols;
+            }
+        }
         // transmitted codewords: random information words through G when a generator matrix is loaded (the reference's -G,
         // src/sim/ldpcsim.cpp:162-165); decoding caller-supplied LLRs has no transmitted word
         kp.tx_var = d_bit_pos_.get();
@@ -715,6 +747,8 @@ namespace b200
             kp.g_col_ptr = d_g_col_ptr_.get(); kp.g_row = d_g_row_.get();
             kp.g_rows = G.mc; kp.g_cols = G.nc; kp.u_words = (G.mc + 31) / 32;
         }
+        if (std::getenv("LDPC_B200_DEBUG"))
+            fprintf(stderr, "[launch] tile kernel: %s\n", kp.early_term ? "early termination" : c.lockstep ? "lock-step" : c.tm ? "half-iteration, TMEM mirror" : "half-iteration");
         launch_kernel(tile_fn(c, kp.early_term != 0), c.ctas, c.threads, c.smem_bytes, s, kp, "tile kernel");
         if (c.residency == LDPC_B200_GLOBAL) release_state(s);
         note_launch(c.fpc, c.threads, c.ctas, c.residency, c.precision, c.smem_bytes);

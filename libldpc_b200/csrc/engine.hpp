@@ -156,6 +156,8 @@ namespace b200
             bool wide;                                // global residency: the 1-CTA-per-SM / 128-register kernel build
             bool idx16;                               // 16-bit index entries (shared-memory residency with the TMEM mirror)
             uint32_t tm_alloc_cols, tm_cols_per_warp, tm_vn_off;
+            bool lockstep;                            // fixed iterations run the lock-step kernel (its gather addresses and descriptors fit)
+            uint32_t tm_idx_off;                      // lock-step kernel: column of the gather addresses inside a warp window
         };
         Config choose(int precision, int alg, uint64_t n_frames);
         const SegLayout &get_seg_layout(int lanes, int threads, int isz = 4);

@@ -150,6 +150,39 @@ namespace b200
     __device__ __forceinline__ void tm_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
     __device__ __forceinline__ void tm_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+    // Lock-step kernel (TM, ET = false): every thread keeps the shared-memory address of each gather of its tasks in its TMEM
+    // lane.  A task of degree D owns W = D rounded up to a power of two columns (one tcgen05.ld.32x32b.xW); the generic-degree
+    // bodies (checks above 8, variables above 16 or of degree 0) own none and keep reading the index tables.
+    __host__ __device__ constexpr int ls_idx_cols(bool check, int deg)
+    {
+        if (check ? (deg < 2 || deg > 8) : (deg < 1 || deg > 16)) return 0;
+        int w = 1;
+        while (w < deg) w <<= 1;
+        return w;
+    }
+    // segment descriptors the lock-step kernel takes from its parameters (K4Params::ls_seg): check lists, then variable lists
+    constexpr int K4_LS_SEGS = 128;
+    template <int D> __device__ __forceinline__ void tm_ld_idx(uint32_t taddr, uint32_t (&e)[D])
+    {
+        constexpr int W = ls_idx_cols(false, D);
+        uint32_t w[W];
+        if constexpr (W == 1) asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(w[0]) : "r"(taddr) : "memory");
+        else if constexpr (W == 2) asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(w[0]), "=r"(w[1]) : "r"(taddr) : "memory");
+        else if constexpr (W == 4)
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]) : "r"(taddr) : "memory");
+        else if constexpr (W == 8)
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                         : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]), "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7]) : "r"(taddr) : "memory");
+        else
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                         : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]), "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7]),
+                           "=r"(w[8]), "=r"(w[9]), "=r"(w[10]), "=r"(w[11]), "=r"(w[12]), "=r"(w[13]), "=r"(w[14]), "=r"(w[15])
+                         : "r"(taddr) : "memory");
+#pragma unroll
+        for (int k = 0; k < D; ++k) e[k] = w[k];
+    }
+    __device__ __forceinline__ void tm_st1(uint32_t taddr, uint32_t v) { asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr), "r"(v) : "memory"); }
+
     // compile-time loop: f(std::integral_constant<int, 0>) ... f(std::integral_constant<int, N-1>)
     template <typename F, int... K>
     __device__ __forceinline__ void static_for_impl(F &&f, std::integer_sequence<int, K...>) { (f(std::integral_constant<int, K>{}), ...); }
@@ -257,6 +290,12 @@ namespace b200
         // TMEM mirror (TM kernels): columns allocated per CTA (power of two >= 32), columns per warp window,
         // column offset of the variable-side (channel LLR) part inside a warp window
         uint32_t tm_alloc_cols, tm_cols_per_warp, tm_vn_off;
+        // lock-step kernel (TM, ET = false): column offset of the gather addresses inside a warp window (ls_idx_cols), and the
+        // segment descriptors of SegLayout in the parameter bank -- check lists at [warp * cn_max_segs], then variable lists at
+        // [warps * cn_max_segs + warp * vn_max_segs] -- so that a warp reads them as uniform values, not through shared memory.
+        // The last word of a warp's first variable descriptor (0 in SegLayout) holds the number of its check-side address columns.
+        uint32_t tm_idx_off;
+        uint32_t ls_seg[4 * K4_LS_SEGS];
     };
 
     // raw value of smaller magnitude (min-sum keeps raw values; magnitude and sign are fixed at the store)
@@ -463,6 +502,19 @@ namespace b200
 #pragma unroll
             for (int e = 0; e < VEC; ++e) bits |= par[e] ? (1u << e) : 0u;
             return bits;
+        }
+        // lock-step kernel: nx holds this node's gather addresses (shared-memory byte addresses: run() with out_sub = 0 and no
+        // index load); those of the next task (TMEM columns ti_next) are loaded while this one runs.  The wait of the c2v mirror
+        // load covers them; the first check phase of a batch reads no mirror and waits at the end of the task.
+        template <int CSRC>
+        static __device__ __forceinline__ void run_ls(uint32_t (&nx)[D], uint32_t ti_next, bool more, P c2v0, uint32_t tc)
+        {
+            uint32_t ga[D];
+#pragma unroll
+            for (int k = 0; k < D; ++k) ga[k] = nx[k];
+            if (more) tm_ld_idx<D>(ti_next, nx);
+            run<CSRC, true, false>(P(0), c2v0, ga, P(0), false, tc, 0u);
+            if constexpr (CSRC == 4) tm_wait_ld();
         }
     };
 
@@ -682,6 +734,15 @@ namespace b200
             }
             return acc;
         }
+        // lock-step kernel: gather addresses in nx, the next task's loaded from TMEM columns ti_next meanwhile (the caller waits)
+        static __device__ __forceinline__ V run_ls(uint32_t (&nx)[D], uint32_t ti_next, bool more, V acc)
+        {
+            uint32_t ga[D];
+#pragma unroll
+            for (int k = 0; k < D; ++k) ga[k] = nx[k];
+            if (more) tm_ld_idx<D>(ti_next, nx);
+            return run(P(0), ga, P(0), false, acc);
+        }
     };
     // arbitrary degree (> 8): 16-byte index chunks (chunk q at ip + q*NPW*16)
     template <typename T, typename IdxT, bool SMEM, int LANES>
@@ -791,8 +852,11 @@ namespace b200
             for (int i = tid; i < p.nct; i += nthreads) sts_u16<0>(a_tx + 2 * i, (uint32_t)p.tx_pos[i]);
             for (int i = tid; i < p.n_punct; i += nthreads) sts_u16<0>(a_pu + 2 * i, (uint32_t)p.punct_pos[i]);
             for (int i = tid; i < p.n_short; i += nthreads) sts_u16<0>(a_sh + 2 * i, (uint32_t)p.short_pos[i]);
-            for (int i = tid; i < 4 * p.cn_max_segs * warps; i += nthreads) sts_u32<0>(a_cs + 4 * i, p.cn_seg[i]);
-            for (int i = tid; i < 4 * p.vn_max_segs * warps; i += nthreads) sts_u32<0>(a_vs + 4 * i, p.vn_seg[i]);
+            if constexpr (ET || !TM) // the lock-step kernel takes its descriptors from the parameters
+            {
+                for (int i = tid; i < 4 * p.cn_max_segs * warps; i += nthreads) sts_u32<0>(a_cs + 4 * i, p.cn_seg[i]);
+                for (int i = tid; i < 4 * p.vn_max_segs * warps; i += nthreads) sts_u32<0>(a_vs + 4 * i, p.vn_seg[i]);
+            }
             for (int i = tid; i < (int)(p.cn_idx_bytes >> 2); i += nthreads) sts_u32<0>(a_ci + 4 * i, reinterpret_cast<const uint32_t *>(p.cn_idx)[i]);
             for (int i = tid; i < (int)(p.vn_idx_bytes >> 2); i += nthreads) sts_u32<0>(a_vi + 4 * i, reinterpret_cast<const uint32_t *>(p.vn_idx)[i]);
             c2v = a_c2v; out = a_out; llr = a_llr; cn_seg = a_cs; vn_seg = a_vs; cn_idx = a_ci; vn_idx = a_vi;
@@ -819,6 +883,38 @@ namespace b200
             __syncthreads();
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             tm_w = s_tmem + (((uint32_t)(warp & 3) * 32u) << 16) + (uint32_t)(warp >> 2) * p.tm_cols_per_warp;
+        }
+        if constexpr (TM && !ET)
+        {
+            // The work of a thread is the same in every phase of the launch: write the shared-memory address of each of its
+            // gathers (check side: `out` record + sub, variable side: c2v record + sub) into its TMEM lane once, task after
+            // task in list order (ls_idx_cols columns each).  The index tables were staged above.
+            constexpr int EPC = 16 / ISZ;
+            uint32_t ti = tm_w + p.tm_idx_off;
+            for (int side = 0; side < 2; ++side)
+            {
+                const int ms = side ? p.vn_max_segs : p.cn_max_segs, s0 = (side ? warps * p.cn_max_segs : 0) + warp * ms;
+                const P base = (side ? c2v : out) + sub * 16, tab = side ? vn_idx : cn_idx;
+                for (int s = s0; s < s0 + ms; ++s)
+                {
+                    const uint4 sg = make_uint4(p.ls_seg[4 * s], p.ls_seg[4 * s + 1], p.ls_seg[4 * s + 2], 0u);
+                    if (sg.x == 0) break;
+                    const int deg = (int)(sg.x & 0xFFu), nt = (int)(sg.x >> 16);
+                    const int w = ls_idx_cols(side == 0, deg), st = idx_stride_of(deg, ISZ);
+                    for (int t = 0; t < nt && w > 0; ++t)
+                        for (int k = 0; k < w; ++k, ++ti)
+                        {
+                            uint32_t a = 0;
+                            if (k < deg)
+                            {
+                                const uint32_t o = sg.z + (uint32_t)(st < 16 ? (t * NPW + j) * st + k * ISZ : t * NPW * st + (k / EPC) * NPW * 16 + j * 16 + (k % EPC) * ISZ);
+                                a = base + (ISZ == 4 ? lds_u32<0>(tab + o) : lds_u16<0>(tab + o) << 4);
+                            }
+                            tm_st1(ti, a);
+                        }
+                }
+            }
+            tm_wait_st();
         }
         if (tid < FPC)
         {
@@ -1360,11 +1456,152 @@ namespace b200
             if constexpr (TM && LSRC == 0) tm_wait_st();
         };
 
+
         // The retire / refill event has exactly ONE call site per kernel.  (The event is ~1 k instructions of cold code; inlined at
         // three sites it no longer shared the 32 KB instruction cache with the decode loop and every event paid for instruction
         // fetches from L2.)
         if constexpr (!ET)
         {
+            // ---- the phases of the lock-step kernel: the same bodies, the descriptors read from the parameter bank (uniform) and
+            //      the gather addresses from TMEM (written by the prologue), one task ahead.  CSRC 4 / LSRC 0: first iteration of a
+            //      batch (no old c2v; the channel LLRs are read from shared memory and mirrored) -----------------------------
+            auto cn_phase_ls = [&](auto csrc)
+            {
+                constexpr int CSRC = decltype(csrc)::value;
+                uint32_t tc = tm_w, ti = tm_w + p.tm_idx_off;
+                for (int s = warp * p.cn_max_segs;; ++s)
+                {
+                    const uint4 sg = make_uint4(p.ls_seg[4 * s], p.ls_seg[4 * s + 1], p.ls_seg[4 * s + 2], 0u);
+                    if (sg.x == 0) break;
+                    const int deg = (int)(sg.x & 0xFFu);
+                    int nt = (int)(sg.x >> 16);
+                    P c2v0 = c2v_lane + sg.y;
+#define B200_CN_LS_CASE(D)                                                                                   \
+    case D:                                                                                                  \
+    {                                                                                                        \
+        uint32_t nx[D];                                                                                      \
+        tm_ld_idx<D>(ti, nx);                                                                                \
+        tm_wait_ld();                                                                                        \
+        _Pragma("unroll 1") for (; nt > 0; --nt)                                                             \
+        {                                                                                                    \
+            ti += ls_idx_cols(true, D);                                                                      \
+            Cn4<T, IdxT, SMEM, LANES, ALG, D>::template run_ls<CSRC>(nx, ti, nt > 1, c2v0, tc);              \
+            c2v0 += D * 512;                                                                                 \
+            tc += 4 * D;                                                                                     \
+        }                                                                                                    \
+        break;                                                                                               \
+        }
+                    switch (deg) // warp-uniform
+                    {
+                        B200_CN_LS_CASE(2)
+                        B200_CN_LS_CASE(3)
+                        B200_CN_LS_CASE(4)
+                        B200_CN_LS_CASE(5)
+                        B200_CN_LS_CASE(6)
+                        B200_CN_LS_CASE(7)
+                        B200_CN_LS_CASE(8)
+                    default: // neither mirrored nor in TMEM: index tables and c2v in shared memory
+                    {
+                        const int st = idx_stride_of(deg, ISZ);
+                        P ip = cn_idx + sg.z + j * 16;
+                        for (; nt > 0; --nt)
+                        {
+                            cn4_any<T, IdxT, SMEM, LANES, ALG>(out_sub, c2v0, ip, deg, CSRC == 4 ? VMASK : 0u);
+                            c2v0 += deg * 512;
+                            ip += NPW * st;
+                        }
+                        break;
+                    }
+                    }
+#undef B200_CN_LS_CASE
+                }
+                tm_wait_st();
+            };
+            auto vn_phase_ls = [&](auto lsrc)
+            {
+                constexpr int LSRC = decltype(lsrc)::value;
+                // the variable-side addresses follow the warp's check-side ones: the first variable descriptor's last word holds
+                // the check-side column count (Engine::launch)
+                const int s0 = warps * p.cn_max_segs + warp * p.vn_max_segs;
+                uint32_t tl = tm_w + p.tm_vn_off, ti = tm_w + p.tm_idx_off + p.ls_seg[4 * s0 + 3];
+                for (int s = s0;; ++s)
+                {
+                    const uint4 sg = make_uint4(p.ls_seg[4 * s], p.ls_seg[4 * s + 1], p.ls_seg[4 * s + 2], 0u);
+                    if (sg.x == 0) break;
+                    const int deg = (int)(sg.x & 0xFFu);
+                    int nt = (int)(sg.x >> 16);
+                    P lp = llr_lane + sg.y, op = out_lane + sg.y;
+                    // channel LLR (decoder.cpp:50); from the mirror its wait also covers the gather addresses loaded by the last task
+                    auto channel_llr = [&]() -> V
+                    {
+                        V a;
+                        if constexpr (LSRC == 1) a = TmAcc<T>::ld(tl);
+                        else
+                        {
+                            a = VAcc<SMEM, T, 0>::ld(lp);
+                            TmAcc<T>::st(tl, a);
+                        }
+                        tm_wait_ld();
+                        return a;
+                    };
+                    auto finish = [&](const V &acc)
+                    {
+                        VAcc<SMEM, T, 0>::st(op, acc);
+                        lp += 512;
+                        op += 512;
+                        tl += 4;
+                    };
+#define B200_VN_LS_CASE(D)                                                                                   \
+    case D:                                                                                                  \
+    {                                                                                                        \
+        uint32_t nx[D];                                                                                      \
+        tm_ld_idx<D>(ti, nx);                                                                                \
+        _Pragma("unroll 1") for (; nt > 0; --nt)                                                             \
+        {                                                                                                    \
+            ti += ls_idx_cols(false, D);                                                                     \
+            const V a = channel_llr();                                                                       \
+            finish(Vn4<T, IdxT, SMEM, LANES, D>::run_ls(nx, ti, nt > 1, a));                                 \
+        }                                                                                                    \
+        break;                                                                                               \
+        }
+                    switch (deg)
+                    {
+                    case 0:
+                        for (; nt > 0; --nt) finish(channel_llr());
+                        break;
+                        B200_VN_LS_CASE(1)
+                        B200_VN_LS_CASE(2)
+                        B200_VN_LS_CASE(3)
+                        B200_VN_LS_CASE(4)
+                        B200_VN_LS_CASE(5)
+                        B200_VN_LS_CASE(6)
+                        B200_VN_LS_CASE(7)
+                        B200_VN_LS_CASE(8)
+                        B200_VN_LS_CASE(9)
+                        B200_VN_LS_CASE(10)
+                        B200_VN_LS_CASE(11)
+                        B200_VN_LS_CASE(12)
+                        B200_VN_LS_CASE(13)
+                        B200_VN_LS_CASE(14)
+                        B200_VN_LS_CASE(15)
+                        B200_VN_LS_CASE(16)
+                    default:
+                    {
+                        const int st = idx_stride_of(deg, ISZ);
+                        P ip = vn_idx + sg.z + j * 16;
+                        for (; nt > 0; --nt)
+                        {
+                            finish(vn4_any<T, IdxT, SMEM, LANES>(c2v_sub, ip, deg, channel_llr()));
+                            ip += NPW * st;
+                        }
+                        break;
+                    }
+                    }
+#undef B200_VN_LS_CASE
+                }
+                if constexpr (LSRC == 0) tm_wait_st();
+            };
+
             // Without early termination every frame lane of the CTA is filled by the same event and reaches max_iter in the same
             // iteration, so the CTA decodes in lock-step batches: fill, max_iter x (check phase, barrier, variable phase,
             // barrier), retire -- the event's call site is the top of a batch and nothing is decided per half iteration.  In a
@@ -1378,8 +1615,8 @@ namespace b200
                 {
                     // first iteration of a batch: every old c2v is +0 and the channel LLRs sit in shared memory only (the variable
                     // phase refreshes their mirror); the later ones read the mirror
-                    if (i == 0) cn_phase(std::integral_constant<int, 4>{});
-                    else cn_phase(std::integral_constant<int, 1>{});
+                    if (i == 0) cn_phase_ls(std::integral_constant<int, 4>{});
+                    else cn_phase_ls(std::integral_constant<int, 1>{});
 #ifdef B200_PHASE_TIMING
                     pt1 = clock64();
                     if (lane == 0) s_pt[0][warp] = pt1;
@@ -1389,8 +1626,8 @@ namespace b200
                     pt2 = 0;
                     for (int w = 0; w < warps; ++w) pt2 = max(pt2, s_pt[0][w]);
 #endif
-                    if (i == 0) vn_phase(std::integral_constant<int, 0>{});
-                    else vn_phase(std::integral_constant<int, 1>{});
+                    if (i == 0) vn_phase_ls(std::integral_constant<int, 0>{});
+                    else vn_phase_ls(std::integral_constant<int, 1>{});
 #ifdef B200_PHASE_TIMING
                     const long long pt3 = clock64();
                     if (lane == 0) s_pt[1][warp] = pt3;
